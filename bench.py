@@ -2,6 +2,7 @@
 """bench.py -- restarts/sec of the batched factorize hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2] [--scaling strong|weak]
+                    [--dump-outputs DIR]
 
 Workload (default c3 = BASELINE.json configs[2], the north-star target; it fits one B200): synthetic 50 000 cells x
 2 000 HVG, K = 5..13 x 100 seeds = 900 restarts, solver 'mu' (Frobenius), tol 1e-4, max_iter 1000 -- the reference's
@@ -20,6 +21,8 @@ solve, the all-gather, D2H of all spectra inside the timed region); `with_consen
 cNMF.consensus numerics for every K (Ks sharded over the ranks) with its HBM roofline; `roofline` = the dominant
 kernel (the batched tcgen05 GEMM) from CUDA events inside the timed region (recorded on rank 0); `cpu_baseline` / `cd_default` = the
 reference's own scikit-learn call timed on the host cores.
+`--dump-outputs DIR` writes what the last timed step returned (see --help); inputs are synthetic and seeded, so two
+builds run with the same arguments can be compared output for output.
 `--impl reference` times the reference's CPU implementation (oracle/reference_path.py: the reference's call
 sequence on scikit-learn, float64): one restart of the job table to convergence per step, K cycling through the
 sweep, on the best thread count of a short sweep.
@@ -186,9 +189,13 @@ def run_reference(args, rank, world):
             reference_path.factorize(X, [jobs[i]], "mu", max_iter=3)
         t0 = time.perf_counter()
         for i in range(args.steps):
-            _, it, _ = reference_path.factorize(X, [jobs[args.warmup + i]], "mu")
+            sp, it, _ = reference_path.factorize(X, [jobs[args.warmup + i]], "mu")
             its += it
         dt = time.perf_counter() - t0
+    if args.dump_outputs:                                      # the last step's restart
+        write_outputs(args.dump_outputs, {"spectra": np.asarray(sp[0], np.float64),
+                                          "n_iter": np.array(it, np.float64),
+                                          "spectra_jobs": np.array([pick[-1]], np.float64)})
     val = args.steps / dt
     sample = ("1 restart of the job table per step to convergence (K cycling %s, reference seeds), sklearn "
               "non_negative_factorization MU float64 as cnmf.py:672 calls it; n_iter=%s; thread sweep (6 iterations): %s"
@@ -201,6 +208,32 @@ def run_reference(args, rank, world):
         "cpu_baseline": {"value": val, "unit": "restarts/s", "cores": threads, "kind": "port", "sample": sample},
         "e2e": {"value": val, "unit": "restarts/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }), flush=True)
+
+
+DUMP_BYTES = 64 * 10 ** 6      # --dump-outputs writes at most this much
+
+
+def dump_jobs(ks, n_genes, budget):
+    """Jobs whose spectra --dump-outputs writes: all of them when they fit in `budget` bytes of fp32, else a fixed
+    seeded random subset of whole restarts that does (the same subset for the same job table)."""
+    size = [int(k) * n_genes * 4 for k in ks]
+    if sum(size) <= budget:
+        return list(range(len(ks)))
+    pick, used = [], 0
+    for j in np.random.RandomState(0).permutation(len(ks)):
+        if used + size[j] <= budget:
+            pick.append(int(j))
+            used += size[j]
+    return sorted(pick)
+
+
+def write_outputs(out_dir, arrays):
+    """arrays: name -> float32 / float64 array, written as out_dir/<name>.npy."""
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def consensus_bytes(R, Rk, G, N, G_all, K, lloyd_iters, refit_iters):
@@ -274,9 +307,8 @@ def run_ours(args, rank, world, local):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     sync_all()
     e0.record()
-    n_iter = None
     for _ in range(args.steps):
-        _, n_iter, my_jobs = step_resident()
+        sharded, n_iter, my_jobs = step_resident()
     e1.record()
     sync_all()
     ms = max_over_ranks(e0.elapsed_time(e1))
@@ -285,6 +317,19 @@ def run_ours(args, rank, world, local):
     eng.profile(False)
     launches = eng.launch_count - launches0
     value = n_jobs * args.steps / (ms * 1e-3)
+
+    dump = None
+    if args.dump_outputs:              # what the last timed step returned: spectra of every job, n_iter of every job
+        it_all = torch.zeros(n_jobs, dtype=torch.float64, device=dev)
+        it_all[torch.as_tensor(my_jobs, dtype=torch.long, device=dev)] = torch.as_tensor(
+            np.asarray(n_iter, np.float64), device=dev)
+        if world > 1:
+            dist.all_reduce(it_all)                            # every job belongs to exactly one rank
+        if rank == 0:                                          # the gathered slab is the same on every rank
+            jobs = dump_jobs(ks_all, X.shape[1], DUMP_BYTES - 16 * n_jobs)
+            spectra = sharded.host()
+            dump = {"spectra": np.vstack([spectra[j] for j in jobs]), "n_iter": it_all.cpu().numpy(),
+                    "spectra_jobs": np.asarray(jobs, np.float64)}
 
     # ---------------- factorize + all-gather + consensus for every K (Ks sharded over the ranks) ----------------
     with_consensus = None
@@ -316,7 +361,7 @@ def run_ours(args, rank, world, local):
 
         step_consensus()                                                   # warm-up (allocations, caches)
         sync_all()
-        n_c = min(args.steps, 3)
+        n_c = args.steps
         t_all0 = time.perf_counter()
         acc = [0.0, 0.0, 0.0]
         per_k = {}
@@ -353,9 +398,10 @@ def run_ours(args, rank, world, local):
         step_resident(CD_KW)
         torch.cuda.synchronize(dev)
         t0 = time.perf_counter()
-        _, it_cd, _ = step_resident(CD_KW)
+        for _ in range(args.steps):
+            _, it_cd, _ = step_resident(CD_KW)
         torch.cuda.synchronize(dev)
-        cd_default = {"gpu_value": n_jobs / (time.perf_counter() - t0), "unit": "restarts/s",
+        cd_default = {"gpu_value": n_jobs * args.steps / (time.perf_counter() - t0), "unit": "restarts/s",
                       "n_iter_mean": float(np.mean(it_cd)), "n_iter_max": int(np.max(it_cd))}
 
     # ---------------- end-to-end arm: host buffers through the public call ----------------
@@ -454,9 +500,11 @@ def run_ours(args, rank, world, local):
                 _, its_cd, sec_cd = reference_path.factorize(X64, [job], "cd")
             cd_default.update(cpu_value=1.0 / sec_cd, cpu_cores=threads,
                               note="the reference's DEFAULT solver for beta_loss='frobenius' (coordinate descent, cnmf.py:629-631): "
-                                   "same job table on the GPU (1 step, resident) vs 1 restart (K=%d, n_iter=%d) of the reference's "
-                                   "sklearn call on the host" % (job[0], its_cd[0]))
+                                   "same job table on the GPU (%d steps, resident) vs 1 restart (K=%d, n_iter=%d) of the reference's "
+                                   "sklearn call on the host" % (args.steps, job[0], its_cd[0]))
     out["cd_default"] = cd_default
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     print(json.dumps(out), flush=True)
 
 
@@ -473,7 +521,14 @@ def main():
     ap.add_argument("--no-cd", action="store_true")
     ap.add_argument("--precision", type=str, default="f16x2", choices=["f16x2", "tf32x3", "tf32x3-general", "fp32"],
                     help="f16x2 (default): 2 kind::f16 passes when X is scaled integer counts, else 3 kind::tf32 passes; tf32x3: 2 / 3 kind::tf32 passes")
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy: spectra "
+                         "(the stacked k x genes spectra of the jobs in spectra_jobs: every job of the table, or a fixed "
+                         "seeded subset when they exceed 64 MB), n_iter (of every job the step solved, in job-table "
+                         "order), spectra_jobs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))

@@ -23,6 +23,8 @@ BASELINE.json configs[0] -- 1 000 cells x 500 HVG, K=7, 10 restarts -- in full) 
   fp32dev_k<K>    per restart: rel-L2 between scikit-learn's OWN float32 path and the reference (float64)
                   spectra for the same seed -- a conditioning yardstick for fp32-class implementations
                   (computed with a direct sklearn call; the reference itself always runs float64)
+``path_table.json`` (``python -m oracle.make_golden path_table``) holds the reference's cNMF path table for
+output_dir D and name "run", every path relative to D.
 Everything derives from RandomState seeds, so the script is reproducible bit for bit on the
 same library versions (numpy 2.3.5, scikit-learn 1.9.0, pandas 3.0.2).
 """
@@ -119,7 +121,25 @@ def run_case(tag, spec):
     print(tag, "->", {k: getattr(v, "shape", v) for k, v in out.items()})
 
 
+def write_path_table():
+    """``path_table.json``: the reference's cNMF(output_dir, name="run").paths, relative to output_dir."""
+    import json
+    ref = refshim.load_reference()
+    tmp = tempfile.mkdtemp(prefix="golden_")
+    try:
+        paths = ref.cNMF(output_dir=tmp, name="run").paths
+        table = {key: os.path.relpath(p, tmp) for key, p in paths.items()}
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
+    with open(os.path.join(GOLDEN_DIR, "path_table.json"), "w") as f:
+        json.dump(table, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print("path_table ->", len(table), "entries")
+
+
 if __name__ == "__main__":
     for tag, spec in CASES.items():
         if len(sys.argv) == 1 or tag in sys.argv[1:]:      # `python -m oracle.make_golden sim_kl` regenerates one
             run_case(tag, spec)
+    if len(sys.argv) == 1 or "path_table" in sys.argv[1:]:
+        write_path_table()
