@@ -279,8 +279,7 @@ static int dataset_finish(cnmf_dataset_s* d, cudaStream_t s) {
   if (d->precision == CNMF_PRECISION_TF32X3) {
     // ---- exact-count detection: is X = diag(r) C diag(s) with C integer <= 2048 ?  (column scale first,
     //      then row scale; datasets derived by cnmf_dataset_from_columns arrive with `exact` already decided)
-    static const bool allow_exact = [] { const char* e = std::getenv("CNMF_EXACT"); return !(e && e[0] == '0'); }();
-    if (allow_exact && d->allow_exact && !d->exact && d->n_rows <= 65535 * 64) {
+    if (d->allow_exact && !d->exact && d->n_rows <= 65535 * 64) {
       float* cmin = nullptr;
       float* rmin = nullptr;
       CNMF_TRY(dataset_alloc(d, &cmin, (size_t)d->ld_c));

@@ -4,34 +4,6 @@
 
 namespace cnmf {
 
-// Multiplicative update of the row factor applied in the epilogue of  NUM = F_other * X^T  (north star: "update applied in
-// the GEMM epilogue"; sklearn _nmf.py:535-549, 610-624).  The product tile never leaves the SM: the accumulate warp
-// thread that owns packed row (o + c) of a restart and 128 items holds their numerators in registers, streams the
-// restart's K old factor rows at those items (one broadcast load per row and 4 items for all lanes of the restart),
-// forms den = sum_i Gram[c, i] F[o + i, item] and writes F_out = F * num / den, its two fp16 operand pieces with the
-// power-of-two scale of its 128-item group and -- when gram_part is given -- the K x K Gram partial of the NEW rows.
-// F_in / F_out are different buffers (other threads read the old rows of the restart while this one writes).
-struct FuseW {
-  const float* F_in;      // SK x ld fp32, old values
-  float* F_out;           // SK x ld fp32, new values (rows of converged restarts are copied, pad rows stay zero)
-  void* P_hi;             // SK x ld fp16 pieces of F_out * piece_scale / group scale
-  void* P_mid;
-  float* tile_scale;      // [row * n_groups + item / 128]
-  int n_groups;           // ceil(ld / 128)
-  int ld;
-  const float* piece_scale;   // optional per-item scale folded into the pieces (exact-count datasets), length >= ld
-  const double* gram_in;  // finalised Gram of the OTHER factor, [rid * KMAX*KMAX + c * KMAX + i]
-  const int* row_slot;    // [M] slot of every packed row, -1 for padding rows
-  const int* off;         // [slots]
-  const int* k;           // [slots]
-  const int* rid;         // [slots]
-  const int* done;        // [rid]
-  float l1, l2;           // regularisation (sklearn _nmf.py:611-614)
-  int kmax;               // largest n_components in the batch (<= 16)
-  double* gram_part;      // optional: [(rid * n_tiles + item tile) * 256 + c * KP + i], KP = K rounded up to 4
-  int active;             // 0 = plain product store (this struct is ignored)
-};
-
 struct GemmArgs {
   const float* A_hi;   // M x Kd, row stride lda   (tf32x3: tf32 "hi" piece; fp32 path: the full matrix)
   const float* A_lo;   // tf32 "lo" piece (unused by the fp32 path)
@@ -43,7 +15,6 @@ struct GemmArgs {
   long long c_split_stride;   // elements between consecutive split-K slices of C
   int splits;                 // requested split-K factor
   int splits_effective;       // gemm_effective_splits(Kd, splits): what the kernel will actually write
-  int chain_kb;               // tf32x3: k-blocks (of 32) accumulated in TMEM before draining to registers (0 -> 1)
   int bn;                     // tf32x3: tile width (UMMA N); 0 = choose from (M, N, Kd, splits)
   int b_exact;                // tf32x3: B_hi holds B exactly (tf32-representable values); B_lo unused -> 2 passes
   const float* out_col_scale; // optional: C[:, n] *= out_col_scale[n] (length >= ldc, 16-byte aligned, zero padded)
@@ -54,9 +25,7 @@ struct GemmArgs {
   // f16: the A pieces were divided by a power of two per (row, group of 512 reduction elements); the accumulate warps
   // multiply each drained TMEM chain (128 elements, never straddling a group) by a_tile_scale[m * a_tiles + group]
   const float* a_tile_scale;
-  int a_tiles;                // groups per row = ceil(Kd / group size)
-  int a_group_kb_shift;       // log2(k-blocks per scale group): 3 = groups of 512 elements (default), 1 = groups of 128
-  FuseW fuse;                 // fuse.active: the W-half update runs in the epilogue, C is not written
+  int a_tiles;                // groups per row = ceil(Kd / 512)
 };
 
 // number of non-empty split-K slices for a reduction length Kd (k-blocks of 32 fp32 / 64 fp16 elements = 128 B)
@@ -68,9 +37,7 @@ int gemm_fixed_splits(int Kd, int f16 = 0);
 
 // Choice of the split-K factor (gemm_fixed_splits) and the tile width for the tcgen05 kernel: minimises
 // (waves of the persistent grid) x (tile cost) x (k-blocks per item + pipeline fill) over the tile widths.
-void gemm_plan(int M, int N, int Kd, int sm_count, int* splits, int* bn, int f16 = 0, int b_exact = 0);
-// whether gemm_tf32x3 runs the CTA-pair (cta_group::2, 256-row tiles) kernel for this problem
-bool gemm_uses_pair(int M, int b_exact);
+void gemm_plan(int M, int N, int Kd, int sm_count, int* splits, int* bn, int f16 = 0);
 
 // tcgen05 / TMEM / TMA path (gemm_tf32x3.cu)
 int gemm_tf32x3(const GemmArgs& g, cudaStream_t stream);

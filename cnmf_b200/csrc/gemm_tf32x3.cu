@@ -32,7 +32,6 @@
 #include <cstdint>
 #include <cstdio>
 #include <algorithm>
-#include <cstdlib>
 #include <map>
 #include <mutex>
 #include <tuple>
@@ -53,19 +52,16 @@ constexpr long long WAIT_TIMEOUT_CYCLES = 4000000000LL;   // ~2 s: a dead pipeli
 
 // BEXACT: the B operand is exactly representable in tf32 (e.g. integer counts), so it needs no "lo" piece:
 // 2 MMAs per k-step instead of 3, 64 KB stages (3 of them) instead of 96 KB (2).
-// CTA2: a pair of CTAs (one cluster, two SMs of a TPC) works on a 256 x BN tile with tcgen05.mma.cta_group::2: each CTA
-// stages its own 128 rows of A and HALF of the B tile, so the operand bytes every SM pulls from L2 per MMA cycle drop
-// from 64 KB to 48 KB per k-block -- the feed the 1-CTA kernel is bound by (profiles/r1i_ncu_f16_summary.txt).
-template <int BN, int STAGES, bool BEXACT, bool CTA2 = false, int EPI_BYTES_OVERRIDE = 0>
+template <int BN, int STAGES, bool BEXACT>
 struct SmemLayout {
   static constexpr int A_BYTES = BM * BK * 4;              // 16 KB
-  static constexpr int B_BYTES = (CTA2 ? BN / 2 : BN) * BK * 4;
+  static constexpr int B_BYTES = BN * BK * 4;
   static constexpr int STAGE_BYTES = 2 * A_BYTES + (BEXACT ? 1 : 2) * B_BYTES;
   static constexpr int TILE_BYTES = STAGES * STAGE_BYTES;
   static constexpr int BAR_OFFSET = TILE_BYTES;            // full[STAGES], empty[STAGES], tfull[2], tempty[2]
   static constexpr int TMEM_PTR_OFFSET = BAR_OFFSET + (2 * STAGES + 4) * 8;
   static constexpr int EPI_OFFSET = TMEM_PTR_OFFSET + 16;   // per accumulate warp: 32 x 20-float transpose patch
-  static constexpr int EPI_BYTES = EPI_BYTES_OVERRIDE > 0 ? EPI_BYTES_OVERRIDE : NUM_EPI_WARPS * 32 * 20 * 4;
+  static constexpr int EPI_BYTES = NUM_EPI_WARPS * 32 * 20 * 4;
   static constexpr int TOTAL = EPI_OFFSET + EPI_BYTES;
   static constexpr int DYN_BYTES = TOTAL + 1024;           // slack for manual 1024 B alignment
 };
@@ -107,54 +103,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
       ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1)
       : "memory");
 }
-// ---- CTA-pair (cluster of 2) variants
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// address of the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// both CTAs of a pair load into their OWN shared memory; the transaction bytes are signalled on the LEADER's barrier
-__device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void umma_f16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void umma_tf32_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-// arrives on the barrier at this offset in BOTH CTAs of the pair once the MMAs issued so far have completed
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(static_cast<uint16_t>(3)) : "memory");
-}
-
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
@@ -191,12 +139,11 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
 }
 
 template <bool F16>
-__device__ __forceinline__ uint32_t make_idesc(int bn, int m = BM) {
+__device__ __forceinline__ uint32_t make_idesc(int bn) {
   // cute::UMMA::InstrDescriptor: c=F32 (1<<4), a/b format @7/@10 (TF32 = 2, F16 = 0), K-major A and B, N>>3 @17, M>>4 @24
-  // (M = 256 for cta_group::2: 128 rows in each CTA of the pair)
   const uint32_t fmt = F16 ? 0u : 2u;
   return (1u << 4) | (fmt << 7) | (fmt << 10) | (static_cast<uint32_t>(bn >> 3) << 17) |
-         (static_cast<uint32_t>(m >> 4) << 24);
+         (static_cast<uint32_t>(BM >> 4) << 24);
 }
 
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
@@ -213,260 +160,22 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-// ------------------------------------------------------------------ fused W-half epilogue
-__device__ __forceinline__ void named_bar(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, bool valid) {
-  const int sz = valid ? 16 : 0;                       // src-size 0: the 16 bytes are zero-filled
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(sz) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-
-// shared memory of the fused epilogue (after the pipeline stages and barriers): a staging area of 128 rows x 36 floats per
-// column half, and per accumulate thread its row of the other factor's Gram (16 floats) and of the new Gram (16 doubles)
-constexpr int FUSE_SROW = 36;                                        // floats per staging row (32 items + pad: conflict-free)
-constexpr int FUSE_STAGING_BYTES = 2 * 128 * FUSE_SROW * 4;          // 36 864
-constexpr int FUSE_G_BYTES = 16 * 256 * 4;                           // 16 384
-constexpr int FUSE_GD_BYTES = 16 * 256 * 8;                          // 32 768
-constexpr int FUSE_EPI_BYTES = FUSE_STAGING_BYTES + FUSE_G_BYTES + FUSE_GD_BYTES;
-
-// The multiplicative update of the row factor, applied to the product tile while it is still in registers (struct
-// FuseW in gemm.h).  Thread = packed row (o + c) of a restart x the 128 items of one scale group; acc[] holds the
-// numerators on entry and the new factor values on exit.  The 128 threads that share a column half exchange rows
-// through a shared-memory staging area: per 32-item chunk every thread publishes the OLD values of its row (cp.async
-// straight from global memory), reads the K rows of its restart (den = sum_i Gram[c, i] F[o + i, item]), publishes the
-// NEW values, accumulates its row of the restart's K x K Gram of the new values (fp32 over 16 items, fp64 beyond: the
-// summation granularity of the stand-alone update kernel) and the warp stores its 32 rows of the chunk coalesced.
-// Restarts never straddle a 128-row tile (the engine packs them that way), so every row a thread needs is in the
-// staging area.  All per-thread state that is indexed by the component lives in shared memory, the component loops are
-// rolled (small code, no local memory: with ~200 KB of shared memory per CTA the L1 is too small to hold spills).
-// Afterwards the thread emits the two fp16 operand pieces of its 128 values with the power-of-two scale of the group:
-// the same bits emit_f16_kernel would produce from F_out.
-template <int HALF>
-__device__ __forceinline__ void fused_w_epilogue(float (&acc)[HALF], const FuseW& fz, int M, int mt, int nt, int n_tiles,
-                                                 int q, int half, int lane, const float* __restrict__ out_scale,
-                                                 uint8_t* epi) {
-  static_assert(HALF == 128, "one thread owns one 128-item scale group");
-  constexpr float EPS32 = 1.1920928955078125e-07f;     // np.finfo(np.float32).eps, sklearn _nmf.py:32
-  constexpr float FMIN = 1.17549435e-38f;
-  constexpr int SR = FUSE_SROW;
-  const int r = q * 32 + lane;                          // row inside the 128-row tile
-  const int tid = half * 128 + r;                       // accumulate-thread index 0..255
-  const int grow = mt * BM + r;
-  const int col0 = nt * 256 + half * HALF;              // first item of this thread's group (tile width 256)
-  float* S = reinterpret_cast<float*>(epi) + half * (128 * SR);     // staging of this column half
-  float* Sr = S + r * SR;
-  float* gs = reinterpret_cast<float*>(epi + FUSE_STAGING_BYTES) + tid;                       // gs[i * 256]
-  double* gd = reinterpret_cast<double*>(epi + FUSE_STAGING_BYTES + FUSE_G_BYTES) + tid;      // gd[i * 256]
-  const int bar_id = 1 + half;
-  const int ld = fz.ld;
-
-  int slot = -1;
-  if (grow < M) slot = __ldg(fz.row_slot + grow);
-  int K = 0, o = grow, rid = 0;
-  bool upd = false, cpy = false;
-  if (slot >= 0) {
-    rid = __ldg(fz.rid + slot);
-    K = __ldg(fz.k + slot);
-    o = __ldg(fz.off + slot);
-    if (__ldg(fz.done + rid)) cpy = true; else upd = true;
-  }
-  const int c = grow - o;
-  const int lr0 = o - mt * BM;                          // tile-local row of the restart's first component
-  const int Kl = upd ? K : 0;
-  const bool want_gram = fz.gram_part != nullptr;
-  const bool row_ok = grow < M;
-  const float* pin = fz.F_in + static_cast<long long>(row_ok ? grow : 0) * ld + col0;
-  const uint32_t sr_addr = smem_u32(Sr);
-
-  // old values of the first chunk on their way while the per-thread state is set up
-#pragma unroll
-  for (int t = 0; t < 8; ++t) cp_async16(sr_addr + 16 * t, pin + 4 * t, row_ok && col0 + 4 * t + 3 < ld);
-  for (int i = 0; i < 16; ++i) {
-    gs[i * 256] = (i < Kl) ? static_cast<float>(fz.gram_in[static_cast<long long>(rid) * (KMAX * KMAX) + c * KMAX + i]) : 0.f;
-    gd[i * 256] = 0.0;
-  }
-  if (out_scale) {                                      // per-item scale of the product (exact-count datasets)
-#pragma unroll
-    for (int j = 0; j < HALF; j += 4) {
-      if (col0 + j + 3 < ld) {
-        const float4 sc = *reinterpret_cast<const float4*>(out_scale + col0 + j);
-        acc[j] *= sc.x; acc[j + 1] *= sc.y; acc[j + 2] *= sc.z; acc[j + 3] *= sc.w;
-      }
-    }
-  }
-  float* pout = fz.F_out;
-  const int sub_r = lane >> 3, sub_c = (lane & 7) * 4;  // coalesced store: 4 rows x 128 B per instruction
-
-#pragma unroll
-  for (int ch = 0; ch < 4; ++ch) {                      // 32 items per chunk
-    cp_async_wait_all();
-    named_bar(bar_id, 128);                             // old rows of the chunk are published
-#pragma unroll
-    for (int hh = 0; hh < 2; ++hh) {                    // 16 items at a time (register budget)
-      float2 den[8];
-#pragma unroll
-      for (int t = 0; t < 8; ++t) den[t] = make_float2(0.f, 0.f);
-#pragma unroll 2
-      for (int i = 0; i < Kl; ++i) {                    // summed in component order, like the reference's W @ HHt row
-        const float2 gi = bcast2(gs[i * 256]);
-        const float4* sp = reinterpret_cast<const float4*>(S + (lr0 + i) * SR + hh * 16);
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const float4 w = sp[t];
-          den[2 * t] = fma2(gi, make_float2(w.x, w.y), den[2 * t]);
-          den[2 * t + 1] = fma2(gi, make_float2(w.z, w.w), den[2 * t + 1]);
-        }
-      }
-#pragma unroll
-      for (int t = 0; t < 4; ++t) {
-        const float4 own = *reinterpret_cast<const float4*>(Sr + hh * 16 + 4 * t);
-        const int j = ch * 32 + hh * 16 + 4 * t;
-        const float2 own0 = make_float2(own.x, own.y), own1 = make_float2(own.z, own.w);
-        const float2 num0 = make_float2(acc[j], acc[j + 1]), num1 = make_float2(acc[j + 2], acc[j + 3]);
-        // regularisation terms unconditionally (adding 0 is exact); zero denominators -> eps (sklearn _nmf.py:615)
-        float2 d0 = fma2(bcast2(fz.l2), own0, add2(den[2 * t], bcast2(fz.l1)));
-        float2 d1 = fma2(bcast2(fz.l2), own1, add2(den[2 * t + 1], bcast2(fz.l1)));
-        d0.x = (d0.x < FMIN) ? EPS32 : d0.x; d0.y = (d0.y < FMIN) ? EPS32 : d0.y;
-        d1.x = (d1.x < FMIN) ? EPS32 : d1.x; d1.y = (d1.y < FMIN) ? EPS32 : d1.y;
-        float2 o0 = mul2(own0, div_nr2(num0, d0));
-        float2 o1 = mul2(own1, div_nr2(num1, d1));
-        if (!upd) {                                     // converged restart: carried over unchanged; padding row: zero
-          o0 = cpy ? own0 : make_float2(0.f, 0.f);
-          o1 = cpy ? own1 : make_float2(0.f, 0.f);
-        }
-        acc[j] = o0.x; acc[j + 1] = o0.y; acc[j + 2] = o1.x; acc[j + 3] = o1.y;
-      }
-    }
-    named_bar(bar_id, 128);                             // everybody has read the old rows
-#pragma unroll
-    for (int t = 0; t < 8; ++t)
-      *reinterpret_cast<float4*>(Sr + 4 * t) = make_float4(acc[ch * 32 + 4 * t], acc[ch * 32 + 4 * t + 1],
-                                                           acc[ch * 32 + 4 * t + 2], acc[ch * 32 + 4 * t + 3]);
-    named_bar(bar_id, 128);                             // new rows of the chunk are published
-    if (want_gram) {
-#pragma unroll 2
-      for (int i = 0; i < Kl; ++i) {
-        const float4* sp = reinterpret_cast<const float4*>(S + (lr0 + i) * SR);
-        float2 sa = make_float2(0.f, 0.f), sb = make_float2(0.f, 0.f);   // two 16-item partial sums
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const float4 w = sp[t], w2 = sp[t + 4];
-          const int j = ch * 32 + 4 * t;
-          sa = fma2(make_float2(acc[j], acc[j + 1]), make_float2(w.x, w.y), sa);
-          sa = fma2(make_float2(acc[j + 2], acc[j + 3]), make_float2(w.z, w.w), sa);
-          sb = fma2(make_float2(acc[j + 16], acc[j + 17]), make_float2(w2.x, w2.y), sb);
-          sb = fma2(make_float2(acc[j + 18], acc[j + 19]), make_float2(w2.z, w2.w), sb);
-        }
-        gd[i * 256] += static_cast<double>(sa.x + sa.y) + static_cast<double>(sb.x + sb.y);
-      }
-    }
-    {                                                   // this warp's 32 rows x 32 items, 4 rows x 128 B per instruction
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const int rr = q * 32 + sub_r + 4 * j;
-        const float4 v = *reinterpret_cast<const float4*>(S + rr * SR + sub_c);
-        const int grow2 = mt * BM + rr, gcol = col0 + ch * 32 + sub_c;
-        if (grow2 < M && gcol + 3 < ld) *reinterpret_cast<float4*>(pout + static_cast<long long>(grow2) * ld + gcol) = v;
-      }
-    }
-    named_bar(bar_id, 128);                             // staging free for the next chunk
-    if (ch < 3) {
-#pragma unroll
-      for (int t = 0; t < 8; ++t) {
-        const int cc = (ch + 1) * 32 + 4 * t;
-        cp_async16(sr_addr + 16 * t, pin + cc, row_ok && col0 + cc + 3 < ld);
-      }
-    }
-  }
-
-  if (want_gram) {                                      // the two column halves of a row meet in shared memory
-    named_bar(3, 256);
-    if (half == 0 && upd) {
-      const int KP = (K + 3) & ~3;                      // layout finalize_kernel reads: [c * KP + i]
-      double* dst = fz.gram_part + (static_cast<long long>(rid) * n_tiles + nt) * 256 + c * KP;
-      for (int i = 0; i < KP; ++i) dst[i] = (i < K) ? gd[i * 256] + gd[i * 256 + 128] : 0.0;
-    }
-    named_bar(3, 256);
-  }
-
-  // ---- fp16 operand pieces of the new values, group scale = power of two from the group maximum
-  float m = 0.f;
-  if (fz.piece_scale) {
-#pragma unroll
-    for (int j = 0; j < HALF; j += 4) {
-      float4 ps = make_float4(1.f, 1.f, 1.f, 1.f);
-      if (col0 + j + 3 < ld) ps = *reinterpret_cast<const float4*>(fz.piece_scale + col0 + j);
-      acc[j] *= ps.x; acc[j + 1] *= ps.y; acc[j + 2] *= ps.z; acc[j + 3] *= ps.w;
-    }
-  }
-#pragma unroll
-  for (int j = 0; j < HALF; ++j) m = fmaxf(m, acc[j]);
-  const float sc = f16_group_scale(m);
-  const float inv = 1.f / sc;                           // power of two: exact
-  if (row_ok && col0 < ld) fz.tile_scale[static_cast<long long>(grow) * fz.n_groups + (col0 >> 7)] = sc;
-  __half* ph = static_cast<__half*>(fz.P_hi);
-  __half* pm = static_cast<__half*>(fz.P_mid);
-  uint32_t* Su = reinterpret_cast<uint32_t*>(Sr);
-  const int sub_r8 = lane >> 2, sub_q = lane & 3;       // 8 rows x 64 B per instruction
-#pragma unroll
-  for (int cc = 0; cc < 4; ++cc) {                      // 32 items = 64 B of halves per row and piece
-#pragma unroll
-    for (int pc = 0; pc < 2; ++pc) {
-      __syncwarp();
-#pragma unroll
-      for (int e = 0; e < 16; e += 4) {
-        uint32_t u[4];
-#pragma unroll
-        for (int k2 = 0; k2 < 4; ++k2) {
-          const float x0 = acc[cc * 32 + 2 * (e + k2)] * inv, x1 = acc[cc * 32 + 2 * (e + k2) + 1] * inv;
-          const __half2 h = __floats2half2_rn(x0, x1);
-          if (pc == 0) {
-            u[k2] = *reinterpret_cast<const uint32_t*>(&h);
-          } else {
-            const float2 hf = __half22float2(h);
-            const __half2 md = __floats2half2_rn(x0 - hf.x, x1 - hf.y);
-            u[k2] = *reinterpret_cast<const uint32_t*>(&md);
-          }
-        }
-        *reinterpret_cast<uint4*>(Su + e) = make_uint4(u[0], u[1], u[2], u[3]);
-      }
-      __syncwarp();
-      __half* dstp = pc == 0 ? ph : pm;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int rr = q * 32 + sub_r8 + 8 * j;
-        const uint4 v = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint32_t*>(S + rr * SR) + sub_q * 4);
-        const int grow2 = mt * BM + rr, gcol = col0 + cc * 32 + sub_q * 8;
-        if (grow2 < M && gcol + 7 < ld) *reinterpret_cast<uint4*>(dstp + static_cast<long long>(grow2) * ld + gcol) = v;
-      }
-    }
-  }
-  __syncwarp();
-}
-
 // ------------------------------------------------------------------ the kernel
 // F16 (with BEXACT): operands are fp16 (two pieces of A, one exact B); a k-block is still 128 B per row = 64 elements,
 // a k-step still 32 B = 16 elements (UMMA_K of kind::f16), so the smem / TMA / descriptor byte geometry is unchanged.
 //
-// CTA2: the grid is made of clusters of two CTAs (ranks 0 / 1 = the two SMs of a TPC).  A work item is a 256 x bn tile:
-// rank r stages rows [256 i + 128 r, +128) of both A pieces and rows [r bn/2, +bn/2) of the B tile; rank 0's MMA thread
-// issues tcgen05.mma.cta_group::2 (M = 256) which reads A from each CTA's own shared memory, the two B halves from both,
-// and leaves rows 0-127 of the product in rank 0's TMEM and rows 128-255 in rank 1's.  Barrier protocol (the one of
-// CUTLASS / DeepGEMM 2-SM kernels): `full` lives in rank 0 (both producers arrive on it, both CTAs' TMA bytes are
-// signalled on it), `empty` and `tfull` exist in both CTAs and are arrived by multicast commits, `tempty` lives in
-// rank 0 and is arrived by the accumulate warps of both CTAs.
-template <int BN, int STAGES, bool BEXACT, bool F16, bool CTA2, bool FUSE = false>
-__device__ __forceinline__ void
-gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMap& tmB_hi, const CUtensorMap& tmB_lo,
-          float* __restrict__ C, int M, int N, int ldc, long long c_split_stride,
-          int m_tiles, int n_tiles, int splits, int total_kb, int kb_per_split, int chain_kb, int bn,
-          const float* __restrict__ out_scale, const float* __restrict__ a_tile_scale, int a_tiles, int a_gshift,
-          const FuseW* __restrict__ fz = nullptr) {
+// 320 threads = 10 warps, allocated as 12 (granularity 4): at most 65536 / (12 * 32) = 170 registers per thread --
+// __launch_bounds__ makes ptxas pick 168; a higher __maxnreg__ compiles but cannot launch
+template <int BN, int STAGES, bool BEXACT, bool F16>
+__global__ void __launch_bounds__(NUM_THREADS, 1)
+gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
+                   const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo,
+                   float* __restrict__ C, int M, int N, int ldc, long long c_split_stride,
+                   int m_tiles, int n_tiles, int splits, int total_kb, int kb_per_split, int chain_kb, int bn,
+                   const float* __restrict__ out_scale, const float* __restrict__ a_tile_scale, int a_tiles, int a_gshift) {
   static_assert(!F16 || BEXACT, "the fp16 path exists for exact integer B operands only");
-  static_assert(!FUSE || (F16 && !CTA2 && BN == 256), "the fused W-half epilogue is built for the kind::f16 1-CTA kernel");
-  static_assert(!CTA2 || BEXACT, "the CTA-pair kernel is built for the exact-B (2-pass) forms");
   constexpr int BKE = F16 ? 2 * BK : BK;                        // elements per k-block
-  using L = SmemLayout<BN, STAGES, BEXACT, CTA2, FUSE ? FUSE_EPI_BYTES : 0>;
+  using L = SmemLayout<BN, STAGES, BEXACT>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;     // SWIZZLE_128B needs 1024 B alignment
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -481,43 +190,31 @@ gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMa
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   constexpr uint32_t TMEM_COLS = 2 * BN;                      // two accumulators (power of two: 256 or 512)
-  const uint32_t rank = CTA2 ? cluster_ctarank() : 0u;       // 0 = leader of the pair
-  const int worker = CTA2 ? static_cast<int>(blockIdx.x >> 1) : static_cast<int>(blockIdx.x);
-  const int n_workers = CTA2 ? static_cast<int>(gridDim.x >> 1) : static_cast<int>(gridDim.x);
-  // CTA2: m_tiles counts 256-row tile PAIRS; this CTA's 128-row tile is 2 * (pair) + rank
-
-  if constexpr (CTA2) cluster_sync_all();                     // both CTAs are running before either touches the pair state
+  const int worker = static_cast<int>(blockIdx.x);
+  const int n_workers = static_cast<int>(gridDim.x);
 
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < STAGES; ++s) {
-      mbar_init(full_bar(s), CTA2 ? 2 : 1);                   // CTA2 (used in rank 0): one arrival per producer
+      mbar_init(full_bar(s), 1);
       mbar_init(empty_bar(s), 1);
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(tfull_bar(a), 1);
-      mbar_init(tempty_bar(a), (CTA2 ? 2 : 1) * NUM_EPI_WARPS);   // one arrival per accumulate warp (of both CTAs)
+      mbar_init(tempty_bar(a), NUM_EPI_WARPS);               // one arrival per accumulate warp
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 1) {
-    if constexpr (CTA2) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;"
-                   ::"r"(smem_base + L::TMEM_PTR_OFFSET), "r"(TMEM_COLS) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                   ::"r"(smem_base + L::TMEM_PTR_OFFSET), "r"(TMEM_COLS) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+                 ::"r"(smem_base + L::TMEM_PTR_OFFSET), "r"(TMEM_COLS) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
   __syncthreads();
-  if constexpr (CTA2) cluster_sync_all();                     // the peer's barriers are initialised before anyone arrives
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
   const int items = m_tiles * n_tiles * splits;
-  const int bnl = CTA2 ? bn >> 1 : bn;                        // B rows this CTA stages
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -525,7 +222,7 @@ gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMa
       int stage = 0;
       uint32_t phase = 0;
       for (int w = worker; w < items; w += n_workers) {
-        const int mt = (w % m_tiles) * (CTA2 ? 2 : 1) + static_cast<int>(rank);
+        const int mt = w % m_tiles;
         const int nt = (w / m_tiles) % n_tiles;
         const int z = w / (m_tiles * n_tiles);
         const int kb0 = z * kb_per_split;
@@ -533,37 +230,20 @@ gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMa
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1u, 0);
           const uint32_t st = smem_base + stage * L::STAGE_BYTES;
-          const uint32_t stage_tx = 2u * L::A_BYTES + (BEXACT ? 1u : 2u) * static_cast<uint32_t>(bnl) * BK * 4u;
-          if constexpr (CTA2) {
-            const uint32_t lead_full = mapa_shared(full_bar(stage), 0);
-            if (rank == 0) mbar_arrive_expect_tx(full_bar(stage), 2u * stage_tx);      // both CTAs' bytes
-            tma_load_2d_pair(st, &tmA_hi, lead_full, kb * BKE, mt * BM);
-            tma_load_2d_pair(st + L::A_BYTES, &tmA_lo, lead_full, kb * BKE, mt * BM);
-            tma_load_2d_pair(st + 2 * L::A_BYTES, &tmB_hi, lead_full, kb * BKE, nt * bn + static_cast<int>(rank) * bnl);
-            if (rank != 0) mbar_arrive_cluster(lead_full);
-          } else {
-            mbar_arrive_expect_tx(full_bar(stage), stage_tx);
-            tma_load_2d(st, &tmA_hi, full_bar(stage), kb * BKE, mt * BM);
-            tma_load_2d(st + L::A_BYTES, &tmA_lo, full_bar(stage), kb * BKE, mt * BM);
-            tma_load_2d(st + 2 * L::A_BYTES, &tmB_hi, full_bar(stage), kb * BKE, nt * bn);
-            if constexpr (!BEXACT) tma_load_2d(st + 2 * L::A_BYTES + L::B_BYTES, &tmB_lo, full_bar(stage), kb * BKE, nt * bn);
-          }
-          if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-        }
-      }
-      if constexpr (CTA2) {
-        // the MMA thread's last commits arrive on this CTA's `empty` barriers from the other SM: see every slot
-        // released before this CTA may retire its shared memory
-        for (int i = 0; i < STAGES; ++i) {
-          mbar_wait(empty_bar(stage), phase ^ 1u, 0);
+          const uint32_t stage_tx = 2u * L::A_BYTES + (BEXACT ? 1u : 2u) * static_cast<uint32_t>(bn) * BK * 4u;
+          mbar_arrive_expect_tx(full_bar(stage), stage_tx);
+          tma_load_2d(st, &tmA_hi, full_bar(stage), kb * BKE, mt * BM);
+          tma_load_2d(st + L::A_BYTES, &tmA_lo, full_bar(stage), kb * BKE, mt * BM);
+          tma_load_2d(st + 2 * L::A_BYTES, &tmB_hi, full_bar(stage), kb * BKE, nt * bn);
+          if constexpr (!BEXACT) tma_load_2d(st + 2 * L::A_BYTES + L::B_BYTES, &tmB_lo, full_bar(stage), kb * BKE, nt * bn);
           if (++stage == STAGES) { stage = 0; phase ^= 1u; }
         }
       }
     }
   } else if (warp == 1) {
-    // ===================== MMA issuer (one thread; the leader CTA of a pair) =====================
-    if (lane == 0 && rank == 0) {
-      const uint32_t idesc = make_idesc<F16>(bn, CTA2 ? 2 * BM : BM);   // UMMA N = bn (multiple of 16, <= BN)
+    // ===================== MMA issuer (one thread) =====================
+    if (lane == 0) {
+      const uint32_t idesc = make_idesc<F16>(bn);               // UMMA N = bn (multiple of 16, <= BN)
       int stage = 0;
       uint32_t phase = 0;
       int buf = 0;
@@ -589,15 +269,7 @@ gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMa
             for (int k = 0; k < BK / UMMA_K; ++k) {
               const uint64_t koff = static_cast<uint64_t>((k * UMMA_K * 4) >> 4);   // +32 B per k-step inside the swizzle row
               const uint32_t acc0 = (kb > c0 || k > 0) ? 1u : 0u;
-              if constexpr (CTA2) {
-                if constexpr (F16) {
-                  umma_f16_pair(tmem_d, a_lo + koff, b_hi + koff, idesc, acc0);     // small terms first
-                  umma_f16_pair(tmem_d, a_hi + koff, b_hi + koff, idesc, 1u);
-                } else {
-                  umma_tf32_pair(tmem_d, a_lo + koff, b_hi + koff, idesc, acc0);
-                  umma_tf32_pair(tmem_d, a_hi + koff, b_hi + koff, idesc, 1u);
-                }
-              } else if constexpr (F16) {
+              if constexpr (F16) {
                 umma_f16(tmem_d, a_lo + koff, b_hi + koff, idesc, acc0);    // small terms first
                 umma_f16(tmem_d, a_hi + koff, b_hi + koff, idesc, 1u);
               } else {
@@ -606,19 +278,10 @@ gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMa
                 umma_tf32(tmem_d, a_hi + koff, b_hi + koff, idesc, 1u);
               }
             }
-            // smem slot is free once these MMAs have read it (CTA2: in both CTAs)
-            if constexpr (CTA2) umma_commit_pair(empty_bar(stage)); else umma_commit(empty_bar(stage));
+            umma_commit(empty_bar(stage));                       // smem slot is free once these MMAs have read it
             if (++stage == STAGES) { stage = 0; phase ^= 1u; }
           }
-          // chain complete -> accumulate warps (CTA2: of both CTAs)
-          if constexpr (CTA2) umma_commit_pair(tfull_bar(buf)); else umma_commit(tfull_bar(buf));
-          if (++buf == 2) { buf = 0; buf_phase ^= 1u; }
-        }
-      }
-      if constexpr (CTA2) {
-        // every chain has been drained by both CTAs before the leader lets go of its barriers
-        for (int i = 0; i < 2; ++i) {
-          mbar_wait(tempty_bar(buf), buf_phase ^ 1u, 1);
+          umma_commit(tfull_bar(buf));                           // chain complete -> accumulate warps
           if (++buf == 2) { buf = 0; buf_phase ^= 1u; }
         }
       }
@@ -633,7 +296,7 @@ gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMa
     int buf = 0;
     uint32_t buf_phase = 0;
     for (int w = worker; w < items; w += n_workers) {
-      const int mt = (w % m_tiles) * (CTA2 ? 2 : 1) + static_cast<int>(rank);
+      const int mt = w % m_tiles;
       const int nt = (w / m_tiles) % n_tiles;
       const int z = w / (m_tiles * n_tiles);
       const int kb0 = z * kb_per_split;
@@ -666,16 +329,8 @@ gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMa
         }
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) {                                // one arrival per warp, on the leader's barrier
-          if constexpr (CTA2) mbar_arrive_cluster(mapa_shared(tempty_bar(buf), 0));
-          else mbar_arrive(tempty_bar(buf));
-        }
+        if (lane == 0) mbar_arrive(tempty_bar(buf));    // one arrival per warp
         if (++buf == 2) { buf = 0; buf_phase ^= 1u; }
-      }
-      if constexpr (FUSE) {
-        // W-half update applied to the tile in registers; the product itself is never stored (gemm.h, struct FuseW)
-        fused_w_epilogue<HALF>(acc, *fz, M, mt, nt, n_tiles, q, half, lane, out_scale, smem_gen + L::EPI_OFFSET);
-        continue;
       }
       // Epilogue.  A thread owns one output row, so a direct store touches 32 rows x 16 B per instruction (32 cache
       // lines: the LSU, not the tensor pipe, then paces short tiles -- the 720-tile W half ran at 0.76 of the MMA rate
@@ -716,51 +371,10 @@ gemm_body(const CUtensorMap& tmA_hi, const CUtensorMap& tmA_lo, const CUtensorMa
 
   tc_fence_before();
   __syncthreads();
-  if constexpr (CTA2) cluster_sync_all();       // neither CTA retires while the other may still signal it
   if (warp == 1) {
     tc_fence_after();
-    if constexpr (CTA2)
-      asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
-    else
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
   }
-}
-
-// 320 threads = 10 warps, allocated as 12 (granularity 4): at most 65536 / (12 * 32) = 170 registers per thread --
-// __launch_bounds__ makes ptxas pick 168; a higher __maxnreg__ compiles but cannot launch
-template <int BN, int STAGES, bool BEXACT, bool F16>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
-                   const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo,
-                   float* __restrict__ C, int M, int N, int ldc, long long c_split_stride,
-                   int m_tiles, int n_tiles, int splits, int total_kb, int kb_per_split, int chain_kb, int bn,
-                   const float* __restrict__ out_scale, const float* __restrict__ a_tile_scale, int a_tiles, int a_gshift) {
-  gemm_body<BN, STAGES, BEXACT, F16, false>(tmA_hi, tmA_lo, tmB_hi, tmB_lo, C, M, N, ldc, c_split_stride, m_tiles, n_tiles,
-                                            splits, total_kb, kb_per_split, chain_kb, bn, out_scale, a_tile_scale, a_tiles,
-                                            a_gshift);
-}
-
-// NUM = F_other * X^T with the multiplicative update of the row factor in the epilogue (kind::f16, 256-wide tiles, no split-K)
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-gemm_fused_w_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
-                    const __grid_constant__ CUtensorMap tmB_hi, int M, int N,
-                    int m_tiles, int n_tiles, int total_kb, const float* __restrict__ out_scale,
-                    const float* __restrict__ a_tile_scale, int a_tiles, int a_gshift, const __grid_constant__ FuseW fz) {
-  gemm_body<256, 2, true, true, false, true>(tmA_hi, tmA_lo, tmB_hi, tmB_hi, nullptr, M, N, 0, 0, m_tiles, n_tiles, 1, total_kb,
-                                             total_kb + (total_kb & 1), 2, 256, out_scale, a_tile_scale, a_tiles, a_gshift, &fz);
-}
-
-// the CTA-pair form: clusters of two CTAs, m_tiles = number of 256-row tile pairs
-template <int BN, int STAGES, bool F16>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
-gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
-                 const __grid_constant__ CUtensorMap tmB_hi,
-                 float* __restrict__ C, int M, int N, int ldc, long long c_split_stride,
-                 int m_tiles, int n_tiles, int splits, int total_kb, int kb_per_split, int chain_kb, int bn,
-                 const float* __restrict__ out_scale, const float* __restrict__ a_tile_scale, int a_tiles, int a_gshift) {
-  gemm_body<BN, STAGES, true, F16, true>(tmA_hi, tmA_lo, tmB_hi, tmB_hi, C, M, N, ldc, c_split_stride, m_tiles, n_tiles,
-                                         splits, total_kb, kb_per_split, chain_kb, bn, out_scale, a_tile_scale, a_tiles,
-                                         a_gshift);
 }
 
 // ------------------------------------------------------------------ host side
@@ -820,24 +434,6 @@ int make_map(CUtensorMap* map, const float* ptr, int rows, int cols, int ld, int
   return 0;
 }
 
-static int env_int(const char* name, int dflt) {
-  const char* e = std::getenv(name);
-  return e ? std::atoi(e) : dflt;
-}
-
-// k-blocks per TMEM accumulation chain: at most 16 MMAs between drains (general: 1 k-block = 12 MMAs,
-// exact-B: 2 k-blocks = 16 MMAs; with 8 MMAs per chain the drain, not the tensor pipe, paced the kernel)
-template <bool BEXACT, bool F16>
-static int pick_chain_kb(const GemmArgs& g) {
-  int chain_kb = g.chain_kb;
-  if (chain_kb <= 0) {
-    static const int env_chain = [] { const int v = env_int("CNMF_CHAIN_KB", 0); return v >= 1 ? v : 0; }();   // tuning knob
-    chain_kb = env_chain > 0 ? env_chain : (BEXACT ? 2 : 1);
-  }
-  if (F16) chain_kb = 2;     // scale groups of 512 elements = 8 k-blocks: chains of 2 never straddle one
-  return chain_kb;
-}
-
 template <int BN, int STAGES, bool BEXACT, bool F16>
 int launch(const GemmArgs& g, cudaStream_t stream) {
   using L = SmemLayout<BN, STAGES, BEXACT>;
@@ -866,10 +462,6 @@ int launch(const GemmArgs& g, cudaStream_t stream) {
       }
     }
   }
-  {
-    static const int env_bn = env_int("CNMF_GEMM_BN", 0);
-    if (env_bn >= 16 && env_bn <= BN && env_bn % 16 == 0) bn = env_bn;
-  }
   if ((rc = make_map(&mBh, g.B_hi, g.N, g.Kd, g.ldb, bn, F16))) return rc;
   if ((rc = make_map(&mBl, BEXACT ? g.B_hi : g.B_lo, g.N, g.Kd, g.ldb, bn, F16))) return rc;
 
@@ -890,104 +482,13 @@ int launch(const GemmArgs& g, cudaStream_t stream) {
   }
   const int items = m_tiles * n_tiles * splits;
   const int grid = items < sms ? items : sms;
-  const int chain_kb = pick_chain_kb<BEXACT, F16>(g);
+  // k-blocks per TMEM accumulation chain: at most 16 MMAs between drains (general: 1 k-block = 12 MMAs,
+  // exact-B and f16: 2 k-blocks = 16 MMAs; with 8 MMAs per chain the drain, not the tensor pipe, paced the kernel).
+  // f16 scale groups of 512 elements = 8 k-blocks (a_gshift = 3): chains of 2 never straddle one.
+  const int chain_kb = BEXACT ? 2 : 1;
   kern<<<grid, NUM_THREADS, L::DYN_BYTES, stream>>>(mAh, mAl, mBh, mBl, g.C, g.M, g.N, g.ldc, g.c_split_stride,
                                                     m_tiles, n_tiles, splits, total_kb, kb_per_split,
-                                                    chain_kb, bn, g.out_col_scale, g.a_tile_scale, g.a_tiles,
-                                                    g.a_group_kb_shift > 0 ? g.a_group_kb_shift : 3);
-  CNMF_CUDA_CHECK(cudaGetLastError());
-  return 0;
-}
-
-// fused W-half launch: 128 x 256 tiles, the whole reduction in one item (no split-K), kind::f16
-int launch_fused_w(const GemmArgs& g, cudaStream_t stream) {
-  using L = SmemLayout<256, 2, true, false, FUSE_EPI_BYTES>;     // 2 stages of 64 KB leave room for the epilogue's state
-  static_assert(L::DYN_BYTES <= 227 * 1024, "fused epilogue state does not fit the shared memory of an SM");
-  CUtensorMap mAh, mAl, mBh;
-  int rc;
-  if ((rc = make_map(&mAh, g.A_hi, g.M, g.Kd, g.lda, BM, true))) return rc;
-  if ((rc = make_map(&mAl, g.A_lo, g.M, g.Kd, g.lda, BM, true))) return rc;
-  if ((rc = make_map(&mBh, g.B_hi, g.N, g.Kd, g.ldb, 256, true))) return rc;
-  int dev = 0, sms = 0;
-  CNMF_CUDA_CHECK(cudaGetDevice(&dev));
-  CNMF_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const int m_tiles = (g.M + BM - 1) / BM, n_tiles = (g.N + 255) / 256;
-  const int total_kb = (g.Kd + 2 * BK - 1) / (2 * BK);
-  static bool attr_set[64] = {};
-  if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    CNMF_CUDA_CHECK(cudaFuncSetAttribute(gemm_fused_w_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L::DYN_BYTES));
-    if (dev >= 0 && dev < 64) attr_set[dev] = true;
-  }
-  const int items = m_tiles * n_tiles;
-  const int grid = items < sms ? items : sms;
-  gemm_fused_w_kernel<<<grid, NUM_THREADS, L::DYN_BYTES, stream>>>(mAh, mAl, mBh, g.M, g.N, m_tiles, n_tiles, total_kb,
-                                                                   g.out_col_scale, g.a_tile_scale, g.a_tiles,
-                                                                   g.a_group_kb_shift > 0 ? g.a_group_kb_shift : 3, g.fuse);
-  CNMF_CUDA_CHECK(cudaGetLastError());
-  return 0;
-}
-
-// CTA-pair launch (exact-B forms): 256 x bn tiles, one cluster of two CTAs per tile, 4 stages of 48 KB
-template <int BN, int STAGES, bool F16>
-int launch_pair(const GemmArgs& g, cudaStream_t stream) {
-  using L = SmemLayout<BN, STAGES, true, true>;
-  static_assert(L::DYN_BYTES <= 227 * 1024, "CTA-pair stages do not fit the shared memory of an SM");
-  constexpr int BKE = F16 ? 2 * BK : BK;
-  CUtensorMap mAh, mAl, mBh;
-  int rc;
-  if ((rc = make_map(&mAh, g.A_hi, g.M, g.Kd, g.lda, BM, F16))) return rc;
-  if ((rc = make_map(&mAl, g.A_lo, g.M, g.Kd, g.lda, BM, F16))) return rc;
-  int dev = 0, sms = 0;
-  CNMF_CUDA_CHECK(cudaGetDevice(&dev));
-  CNMF_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const int m_pairs = (g.M + 2 * BM - 1) / (2 * BM);
-  int bn = g.bn;
-  if (bn <= 0 || bn > BN || bn % 16 != 0) bn = g.N <= BN ? ((g.N + 15) / 16) * 16 : BN;
-  {
-    static const int env_bn = env_int("CNMF_GEMM_BN", 0);
-    if (env_bn >= 16 && env_bn <= BN && env_bn % 16 == 0) bn = env_bn;
-  }
-  if ((rc = make_map(&mBh, g.B_hi, g.N, g.Kd, g.ldb, bn / 2, F16))) return rc;    // each CTA stages half of the B tile
-
-  const int n_tiles = (g.N + bn - 1) / bn;
-  const int total_kb = (g.Kd + BKE - 1) / BKE;
-  int splits = g.splits < 1 ? 1 : g.splits;
-  if (splits > total_kb) splits = total_kb;
-  int kb_per_split = (total_kb + splits - 1) / splits;
-  if (F16 && (kb_per_split & 1)) ++kb_per_split;
-  splits = (total_kb + kb_per_split - 1) / kb_per_split;
-  if (splits != g.splits_effective) { set_last_error("gemm: splits_effective mismatch (use gemm_effective_splits)"); return -1; }
-
-  auto kern = gemm_pair_kernel<BN, STAGES, F16>;
-  static bool attr_set[64] = {};
-  static int max_clusters[64] = {};
-  const int di = (dev >= 0 && dev < 64) ? dev : 0;
-  if (!attr_set[di]) {
-    CNMF_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::DYN_BYTES));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(sms & ~1);
-    cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = L::DYN_BYTES;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess || n < 1) {
-      cudaGetLastError();
-      n = sms / 2;
-    }
-    max_clusters[di] = n;
-    attr_set[di] = true;
-  }
-  const int items = m_pairs * n_tiles * splits;
-  const int clusters = items < max_clusters[di] ? items : max_clusters[di];
-  const int chain_kb = pick_chain_kb<true, F16>(g);
-  kern<<<2 * clusters, NUM_THREADS, L::DYN_BYTES, stream>>>(mAh, mAl, mBh, g.C, g.M, g.N, g.ldc, g.c_split_stride,
-                                                            m_pairs, n_tiles, splits, total_kb, kb_per_split,
-                                                            chain_kb, bn, g.out_col_scale, g.a_tile_scale, g.a_tiles,
-                                                            g.a_group_kb_shift > 0 ? g.a_group_kb_shift : 3);
+                                                    chain_kb, bn, g.out_col_scale, g.a_tile_scale, g.a_tiles, 3);
   CNMF_CUDA_CHECK(cudaGetLastError());
   return 0;
 }
@@ -1006,21 +507,8 @@ int gemm_fixed_splits(int Kd, int f16) {
   return gemm_effective_splits(Kd, s, f16);
 }
 
-// CTA pairs (cta_group::2): each SM pulls 48 KB instead of 64 KB of operands per k-block from L2.  MEASURED (run r2b,
-// profiles/r2b_gemm_pair_vs_1cta.log): correct (same bits as the 1-CTA kernel) but 0.65x its speed -- 387 vs 608 TFLOP/s on
-// the c2 W half, 487 vs 740 on 4096 x 16384 x 2000.  The 1-CTA kernel already runs at ~0.9 of the MMA rate its two passes
-// allow when timed alone, so the operand feed was not the limiter; what the pair adds is a cross-SM round trip (remote
-// mbarrier arrive + multicast commit) on EVERY 16-MMA accumulation chain, and with chains that short (the TMEM
-// truncation fix) the handshake, not the tensor pipe, paces the pair.  Kept as an opt-in (CNMF_GEMM_PAIR=1).
-bool gemm_uses_pair(int M, int b_exact) {
-  static const int env_pair = env_int("CNMF_GEMM_PAIR", 0);
-  return env_pair != 0 && b_exact && M > BM;
-}
-
-void gemm_plan(int M, int N, int Kd, int sm_count, int* splits_out, int* bn_out, int f16, int b_exact) {
-  const bool pair = gemm_uses_pair(M, b_exact || f16);
-  const int m_tiles = pair ? (M + 2 * BM - 1) / (2 * BM) : (M + BM - 1) / BM;
-  if (pair) sm_count /= 2;                                   // workers are CTA pairs
+void gemm_plan(int M, int N, int Kd, int sm_count, int* splits_out, int* bn_out, int f16) {
+  const int m_tiles = (M + BM - 1) / BM;
   const int bke = f16 ? 2 * BK : BK;
   const int total_kb = (Kd + bke - 1) / bke;
   const int s = gemm_fixed_splits(Kd, f16);
@@ -1061,23 +549,13 @@ int gemm_tf32x3(const GemmArgs& g, cudaStream_t stream) {
                 reinterpret_cast<uintptr_t>(g.B_hi) | reinterpret_cast<uintptr_t>(g.B_lo) |
                 reinterpret_cast<uintptr_t>(g.C) | reinterpret_cast<uintptr_t>(g.out_col_scale)) % 16 == 0,
                "gemm: pointers must be 16-byte aligned");
-  const bool pair = gemm_uses_pair(g.M, g.b_exact);
   if (g.f16) {
     CNMF_REQUIRE(g.b_exact, "gemm: the fp16 path needs an exact B operand");
     CNMF_REQUIRE(g.lda % 8 == 0 && g.ldb % 8 == 0, "gemm: fp16 leading dimensions must be multiples of 8 halves");
     CNMF_REQUIRE(!g.a_tile_scale || g.a_tiles * 512 >= g.Kd, "gemm: a_tiles does not cover the reduction length");
-    CNMF_REQUIRE(g.chain_kb == 0 || g.chain_kb == 2, "gemm: the fp16 path drains chains of 2 k-blocks");
-    if (g.fuse.active) {
-      CNMF_REQUIRE(g.fuse.F_in && g.fuse.F_out && g.fuse.F_in != g.fuse.F_out && g.fuse.P_hi && g.fuse.P_mid &&
-                       g.fuse.tile_scale && g.fuse.gram_in && g.fuse.row_slot && g.fuse.ld % 32 == 0,
-                   "gemm: incomplete fused-update arguments");
-      return launch_fused_w(g, stream);
-    }
-    if (pair) return launch_pair<256, 4, true>(g, stream);
     return launch<256, 3, true, true>(g, stream);
   }
   if (g.b_exact) {
-    if (pair) return launch_pair<256, 4, false>(g, stream);
     return launch<256, 3, true, false>(g, stream);
   }
   return launch<256, 2, false, false>(g, stream);

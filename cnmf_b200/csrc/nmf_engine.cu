@@ -11,7 +11,6 @@
 // (their blocks exit) and the host only polls the flags.
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 #include "engine.h"
@@ -51,7 +50,7 @@ struct GemmPlan {
 // C[z] (SK x N) = A (SK x Kd) * B (N x Kd)^T
 int run_gemm(cnmf_handle_s* h, int precision, const float* A, const float* A_hi, const float* A_lo, int SK, int lda,
              const Operand& B, float* C, int ldc, const GemmPlan& plan, bool exact, const float* out_scale,
-             bool f16, const float* a_tile_scale, cudaStream_t s, int a_group = 512, const FuseW* fuse = nullptr) {
+             bool f16, const float* a_tile_scale, cudaStream_t s) {
   GemmArgs g{};
   g.M = SK; g.N = B.rows; g.Kd = B.cols;
   g.lda = lda; g.ldb = B.ld; g.ldc = ldc;
@@ -71,9 +70,7 @@ int run_gemm(cnmf_handle_s* h, int precision, const float* A, const float* A_hi,
       g.f16 = 1;
       g.B_hi = static_cast<const float*>(B.h16);
       g.a_tile_scale = a_tile_scale;
-      g.a_tiles = (lda + a_group - 1) / a_group;
-      g.a_group_kb_shift = a_group == 128 ? 1 : 3;
-      if (fuse) g.fuse = *fuse;
+      g.a_tiles = (lda + 511) / 512;
     }
     rc = gemm_tf32x3(g, s);
   } else {
@@ -114,27 +111,6 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
   }
   int R = R0, SK = SK0;     // live slots / live packed rows
   const int kp = kmax <= 16 ? 16 : 32;
-  // MU, f16x2, K <= 16, both factors iterated, whole gene reduction in one slice: the W-half update can run in the
-  // epilogue of its own GEMM (gemm.h, struct FuseW) so that the product NUM_r is never materialised.  Parity-green
-  // (same n_iter, same accuracy class) but MEASURED SLOWER than GEMM + separate update kernel (c3: 715 vs 870
-  // restarts/s, run r2f): the epilogue's ~50 k warp-instructions per tile run on the 8 accumulate warps only (2 per
-  // scheduler, 168 registers of which 128 hold the tile) and do not overlap the tensor pipe beyond the two TMEM chain
-  // buffers.  Opt-in with CNMF_FUSE_W=1 until the update runs as a third warp role under the next tile's main loop.
-  static const bool env_fuse_w = [] { const char* e = std::getenv("CNMF_FUSE_W"); return e && e[0] == '1'; }();
-  const bool fuse_w = env_fuse_w && f16 && mu && kp == 16 && io.update_cols && gemm_fixed_splits(v.n_c, 1) == 1;
-  // packing rule of the fused path: a restart never straddles a 128-row GEMM tile (its K rows meet in one CTA's
-  // epilogue); padding rows hold zeros.  The caller's buffers stay in the unpadded layout (off0).
-  auto pack_offsets = [&](const std::vector<int>& kk, std::vector<int>& offs) -> int {
-    int pos = 0;
-    offs.clear();
-    for (int k : kk) {
-      if (fuse_w && (pos % 128) + k > 128) pos = (pos + 127) / 128 * 128;
-      offs.push_back(pos);
-      pos += k;
-    }
-    return pos;
-  };
-  const int SKcap = fuse_w ? ((SK0 + (128 - kmax)) / (128 - kmax + 1)) * 128 + 128 : SK0;   // rows any packing can need
   // block granularity of the streaming kernels, fixed for the whole solve (partial buffers are sized by it)
   // update kernels: 3 blocks of 128 threads per SM resident, a block walks 1-4 tiles -> aim for >= 8 blocks per SM;
   // stand-alone Gram kernel: 1 block/SM resident and a fixed-cost block reduction -> long blocks, about two waves
@@ -164,10 +140,8 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
   double* d_state = static_cast<double*>(h->dev_buf("solve.state", sizeof(double) * 8 * R0));
   double* d_gram = static_cast<double*>(h->dev_buf("solve.gram", sizeof(double) * 2 * R0 * KMAX * KMAX));
   // per-block Gram partials of each factor (summed by the last block of the producing launch)
-  const size_t gpart_elems0 = std::max((size_t)R0 * std::max(gchunks_max, std::max((v.n_r + 1023) / 1024, (v.n_c + 1023) / 1024)),
-                                      fused_part_slots) * kp * kp;
-  const int ntiles_r = (v.n_r + 255) / 256;                 // item tiles of the fused W-half GEMM (one Gram partial each)
-  const size_t gpart_elems = std::max(gpart_elems0, fuse_w ? (size_t)R0 * ntiles_r * kp * kp : (size_t)0);
+  const size_t gpart_elems = std::max((size_t)R0 * std::max(gchunks_max, std::max((v.n_r + 1023) / 1024, (v.n_c + 1023) / 1024)),
+                                     fused_part_slots) * kp * kp;
   double* d_gram_part = static_cast<double*>(h->dev_buf("solve.gram_part", sizeof(double) * 2 * gpart_elems));
   double* d_scal_part = static_cast<double*>(h->dev_buf("solve.scal_part", sizeof(double) * 2 * (size_t)R0 * chunks_cap));
   if (!d_meta || !d_state || !d_gram || !d_gram_part || !d_scal_part) return -2;
@@ -176,7 +150,7 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
   float *NUMr = nullptr, *NUMc = nullptr;
   auto plan_one = [&](int sk, int n, int kd, GemmPlan* pl) {
     if (tf32) {
-      gemm_plan(sk, n, kd, h->sm_count, &pl->splits, &pl->bn, f16 ? 1 : 0, v.exact ? 1 : 0);
+      gemm_plan(sk, n, kd, h->sm_count, &pl->splits, &pl->bn, f16 ? 1 : 0);
     } else {
       pl->splits = gemm_fixed_splits(kd, 0);
       pl->bn = 0;
@@ -190,17 +164,13 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
     return 0;
   };
   plan_gemms();
-  // size the product buffers: the split-K factor depends on the reduction length only, the rows never exceed SKcap
-  // (padded packing of the fused path included)
+  // size the product buffers: the split-K factor depends on the reduction length only, the rows never exceed SK0
   {
-    GemmPlan a, b2;
-    plan_one(SKcap, v.n_r, v.n_c, &a);
-    plan_one(SKcap, v.n_c, v.n_r, &b2);
-    const size_t need_r = (size_t)a.splits * (size_t)SKcap * v.ld_r;
-    const size_t need_c = (size_t)b2.splits * (size_t)SKcap * v.ld_c;
-    NUMr = fuse_w ? nullptr : static_cast<float*>(h->dev_buf("solve.NUMr", sizeof(float) * need_r));
+    const size_t need_r = (size_t)plan_r.splits * (size_t)SK0 * v.ld_r;
+    const size_t need_c = (size_t)plan_c.splits * (size_t)SK0 * v.ld_c;
+    NUMr = static_cast<float*>(h->dev_buf("solve.NUMr", sizeof(float) * need_r));
     NUMc = io.update_cols ? static_cast<float*>(h->dev_buf("solve.NUMc", sizeof(float) * need_c)) : nullptr;
-    if ((!fuse_w && !NUMr) || (io.update_cols && !NUMc)) return -2;
+    if (!NUMr || (io.update_cols && !NUMc)) return -2;
   }
 
   int* d_off = d_meta;             // [slots]
@@ -209,19 +179,7 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
   int* d_done = d_meta + 3 * R0;   // [rid]
   int* d_niter = d_meta + 4 * R0;  // [rid]
   int* d_ticket = d_meta + 5 * R0; // [rid] last-block tickets of the fused update kernels (self-resetting)
-  int* d_rowslot = nullptr;        // fused W half: slot of every packed row (-1 = padding)
-  if (fuse_w) {
-    d_rowslot = static_cast<int*>(h->dev_buf("solve.rowslot", sizeof(int) * (size_t)SKcap));
-    if (!d_rowslot) return -2;
-  }
   auto upload_slots = [&]() -> int {
-    if (fuse_w) {
-      std::vector<int> rs(SKcap, -1);
-      for (int sl = 0; sl < R; ++sl)
-        for (int c = 0; c < s_k[sl]; ++c) rs[s_off[sl] + c] = sl;
-      CNMF_CUDA_CHECK(cudaMemcpyAsync(d_rowslot, rs.data(), sizeof(int) * (size_t)SKcap, cudaMemcpyHostToDevice, s));
-      CNMF_CUDA_CHECK(cudaStreamSynchronize(s));      // rs goes out of scope
-    }
     std::vector<int> hm(3 * R0, 0);
     std::memcpy(hm.data(), s_off.data(), sizeof(int) * R);
     std::memcpy(hm.data() + R0, s_k.data(), sizeof(int) * R);
@@ -247,15 +205,14 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
   float *wFr = io.Fr, *wFr_hi = io.Fr_hi, *wFr_lo = io.Fr_lo, *wFc = io.Fc, *wFc_hi = io.Fc_hi, *wFc_lo = io.Fc_lo;
   float *aFr = nullptr, *aFr_hi = nullptr, *aFr_lo = nullptr, *aFc = nullptr, *aFc_hi = nullptr, *aFc_lo = nullptr;
   float *resFr = nullptr, *resFc = nullptr;   // final factors of restarts that were compacted away (original offsets)
-  float* pongFr = nullptr;                    // fused W half: the epilogue writes the new row factor here, then swap
   bool compacted = false;
 
   auto bm = [&]() { return BatchMeta{d_off, d_k, d_rid, d_done, R, kp}; };
   float* d_rs_r = nullptr;   // f16: power-of-two scales of the Fr / Fc pieces, [packed row][512-element group]
   float* d_rs_c = nullptr;
   if (f16) {
-    d_rs_r = static_cast<float*>(h->dev_buf("solve.rowscale_r", sizeof(float) * (size_t)SKcap * ((v.ld_r + (fuse_w ? 127 : 511)) / (fuse_w ? 128 : 512))));
-    d_rs_c = static_cast<float*>(h->dev_buf("solve.rowscale_c", sizeof(float) * (size_t)SKcap * ((v.ld_c + 511) / 512)));
+    d_rs_r = static_cast<float*>(h->dev_buf("solve.rowscale_r", sizeof(float) * (size_t)SK0 * ((v.ld_r + 511) / 512)));
+    d_rs_c = static_cast<float*>(h->dev_buf("solve.rowscale_c", sizeof(float) * (size_t)SK0 * ((v.ld_c + 511) / 512)));
     if (!d_rs_r || !d_rs_c) return -2;
   }
   // tf32 pieces are written by the update kernels; the fp16 pieces need the row maximum first and come from
@@ -263,15 +220,13 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
   const bool upd_pieces = tf32 && !f16;
   // f16: the Gram-fused update kernels (K <= 16, factor being iterated) emit the fp16 pieces themselves, per 512-column
   // tile; everything else (initial factors, compaction, K > 16) goes through emit_pieces() with one scale per row
-  // scale groups of the Fr pieces: 128 items when the fused GEMM epilogue emits them (one group per thread), else 512
-  const int group_r = fuse_w ? 128 : 512;
-  const int ktiles_r = (v.ld_r + group_r - 1) / group_r, ktiles_c = (v.ld_c + 511) / 512;
+  const int ktiles_r = (v.ld_r + 511) / 512, ktiles_c = (v.ld_c + 511) / 512;
   const bool emit_in_update = f16 && kp == 16 && io.update_cols;
   auto fr = [&]() {
     FactorView f{};
     f.F = wFr; f.F_hi = upd_pieces ? wFr_hi : nullptr; f.F_lo = upd_pieces ? wFr_lo : nullptr;
     f.n = v.n_r; f.ld = v.ld_r; f.piece_scale = v.exact ? v.scale_r : nullptr;
-    if (emit_in_update && !fuse_w) { f.P_hi = wFr_hi; f.P_mid = wFr_lo; f.tile_scale = d_rs_r; f.n_ktiles = ktiles_r; }
+    if (emit_in_update) { f.P_hi = wFr_hi; f.P_mid = wFr_lo; f.tile_scale = d_rs_r; f.n_ktiles = ktiles_r; }
     f.cpb = cpb_r; f.gcpb = gcpb_r;
     return f;
   };
@@ -302,7 +257,7 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
     const int slot = h->prof_begin(s, 8.0 * (double)SK * (double)n, 1);   // fp32 in, two fp16 pieces out
     const int rc = side_is_c
         ? launch_emit_f16(wFc, SK, v.n_c, v.ld_c, v.exact ? v.scale_c : nullptr, wFc_hi, wFc_lo, d_rs_c, ktiles_c, s)
-        : launch_emit_f16(wFr, SK, v.n_r, v.ld_r, v.exact ? v.scale_r : nullptr, wFr_hi, wFr_lo, d_rs_r, ktiles_r, s, group_r);
+        : launch_emit_f16(wFr, SK, v.n_r, v.ld_r, v.exact ? v.scale_r : nullptr, wFr_hi, wFr_lo, d_rs_r, ktiles_r, s);
     h->prof_end(s, slot);
     return rc;
   };
@@ -343,24 +298,7 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
   };
   auto gemm_cols = [&]() -> int {   // NUM_c = Fr * B_cols^T
     return run_gemm(h, p.precision, wFr, wFr_hi, wFr_lo, SK, v.ld_r, v.B_cols, NUMc, v.ld_c, plan_c, v.exact, v.scale_c,
-                    f16, d_rs_r, s, group_r);
-  };
-  // fused W half: Fr <- Fr * (Fc X^T) / (Gram(Fc) Fr) inside the GEMM that forms Fc X^T; leaves the new Fr in pongFr
-  // (swapped in by the caller), its fp16 pieces + group scales in place, and per-tile partials of Gram(Fr)
-  auto gemm_rows_fused = [&](float l1, float l2) -> int {
-    FuseW fz{};
-    fz.F_in = wFr; fz.F_out = pongFr;
-    fz.P_hi = wFr_hi; fz.P_mid = wFr_lo; fz.tile_scale = d_rs_r; fz.n_groups = ktiles_r; fz.ld = v.ld_r;
-    fz.piece_scale = v.exact ? v.scale_r : nullptr;
-    fz.gram_in = d_gramC;
-    fz.row_slot = d_rowslot; fz.off = d_off; fz.k = d_k; fz.rid = d_rid; fz.done = d_done;
-    fz.l1 = l1; fz.l2 = l2; fz.kmax = kmax;
-    fz.gram_part = d_gpartR;
-    fz.active = 1;
-    GemmPlan pl = plan_r;
-    pl.splits = 1; pl.bn = 256;
-    return run_gemm(h, p.precision, wFc, wFc_hi, wFc_lo, SK, v.ld_c, v.B_rows, nullptr, v.ld_r, pl, v.exact, v.scale_r,
-                    f16, d_rs_c, s, 512, &fz);
+                    f16, d_rs_r, s);
   };
 
   // gathers `cnt` restarts' rows: dst[dst_off[i] ..] <- src[src_off[i] ..].  Index triples go through a pinned
@@ -415,23 +353,17 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
 
   std::vector<int> h_done(R0, 0);
   // Drop converged restarts from the packed arrays when that saves a 128-row GEMM tile (or >= 1/8 of the rows).
-  auto maybe_compact = [&](bool force = false) -> int {
+  auto maybe_compact = [&]() -> int {
     if (!io.update_cols) return 0;
-    if (!force) {
-      int live_rows = 0;
-      for (int sl = 0; sl < R; ++sl)
-        if (!h_done[s_rid[sl]]) live_rows += s_k[sl];
-      if (live_rows == SK || live_rows == 0) return 0;
-      std::vector<int> lk, lo;
-      for (int sl = 0; sl < R; ++sl)
-        if (!h_done[s_rid[sl]]) lk.push_back(s_k[sl]);
-      const int new_rows = pack_offsets(lk, lo);            // rows of the packed live set (padding included)
-      const bool saves_tile = (new_rows + 127) / 128 < (SK + 127) / 128;
-      if (!saves_tile && new_rows > SK - SK / 8) return 0;
-    }
+    int live_rows = 0;
+    for (int sl = 0; sl < R; ++sl)
+      if (!h_done[s_rid[sl]]) live_rows += s_k[sl];
+    if (live_rows == SK || live_rows == 0) return 0;
+    const bool saves_tile = (live_rows + 127) / 128 < (SK + 127) / 128;
+    if (!saves_tile && live_rows > SK - SK / 8) return 0;
     if (!mu) CNMF_TRY(cd_final_error());    // restarts leaving the packed arrays get their ||X - WH||_F now
     if (!aFr) {
-      const size_t nr = (size_t)SKcap * v.ld_r, nc = (size_t)SKcap * v.ld_c;
+      const size_t nr = (size_t)SK0 * v.ld_r, nc = (size_t)SK0 * v.ld_c;
       aFr = static_cast<float*>(h->dev_buf("solve.alt.Fr", nr * 4));
       aFc = static_cast<float*>(h->dev_buf("solve.alt.Fc", nc * 4));
       resFr = static_cast<float*>(h->dev_buf("solve.res.Fr", nr * 4));
@@ -445,21 +377,16 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
         if (!aFr_hi || !aFr_lo || !aFc_hi || !aFc_lo) return -2;
       }
     }
-    std::vector<int> f_src, f_dst, f_k, l_src, l_dst, l_k, n_off, n_k, n_rid;
+    std::vector<int> f_src, f_dst, f_k, l_src, l_dst, l_k, l_rid;
+    int pos = 0;
     for (int sl = 0; sl < R; ++sl) {
       const int rid = s_rid[sl];
       if (h_done[rid]) {
         f_src.push_back(s_off[sl]); f_dst.push_back(off0[rid]); f_k.push_back(s_k[sl]);
       } else {
-        l_src.push_back(s_off[sl]); l_k.push_back(s_k[sl]);
-        n_k.push_back(s_k[sl]); n_rid.push_back(rid);
+        l_src.push_back(s_off[sl]); l_dst.push_back(pos); l_k.push_back(s_k[sl]); l_rid.push_back(rid);
+        pos += s_k[sl];
       }
-    }
-    const int pos = pack_offsets(l_k, l_dst);
-    n_off = l_dst;
-    if (fuse_w) {      // padding rows of the new packing must read as zeros
-      CNMF_CUDA_CHECK(cudaMemsetAsync(aFr, 0, (size_t)SKcap * v.ld_r * 4, s));
-      CNMF_CUDA_CHECK(cudaMemsetAsync(aFc, 0, (size_t)SKcap * v.ld_c * 4, s));
     }
     CNMF_TRY(gather(wFr, resFr, f_src, f_dst, f_k, v.ld_r));       // finished restarts -> result slabs
     CNMF_TRY(gather(wFc, resFc, f_src, f_dst, f_k, v.ld_c));
@@ -473,11 +400,11 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
     }
     std::swap(wFr, aFr); std::swap(wFr_hi, aFr_hi); std::swap(wFr_lo, aFr_lo);
     std::swap(wFc, aFc); std::swap(wFc_hi, aFc_hi); std::swap(wFc_lo, aFc_lo);
-    R = (int)n_k.size();
+    R = (int)l_k.size();
     SK = pos;
-    std::copy(n_off.begin(), n_off.end(), s_off.begin());
-    std::copy(n_k.begin(), n_k.end(), s_k.begin());
-    std::copy(n_rid.begin(), n_rid.end(), s_rid.begin());
+    std::copy(l_dst.begin(), l_dst.end(), s_off.begin());
+    std::copy(l_k.begin(), l_k.end(), s_k.begin());
+    std::copy(l_rid.begin(), l_rid.end(), s_rid.begin());
     CNMF_TRY(upload_slots());      // synchronises the stream: the gather ring can be reused
     gslot = 0;
     plan_gemms();
@@ -498,21 +425,6 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
 
   const float l1W = (float)p.l1_reg_W, l2W = (float)p.l2_reg_W, l1H = (float)p.l1_reg_H, l2H = (float)p.l2_reg_H;
   int it = 0;
-  if (fuse_w) {
-    // into the padded packing (the "alt" set).  The caller's buffers, now the other half of the ping-pong, are too small
-    // for a later re-packing (SK0 rows, no padding): the ping-pong gets a second set of its own, and the fused epilogue
-    // its output buffer
-    CNMF_TRY(maybe_compact(true));
-    const size_t nr = (size_t)SKcap * v.ld_r, nc = (size_t)SKcap * v.ld_c;
-    aFr = static_cast<float*>(h->dev_buf("solve.altB.Fr", nr * 4));
-    aFr_hi = static_cast<float*>(h->dev_buf("solve.altB.Fr_hi", nr * 4));
-    aFr_lo = static_cast<float*>(h->dev_buf("solve.altB.Fr_lo", nr * 4));
-    aFc = static_cast<float*>(h->dev_buf("solve.altB.Fc", nc * 4));
-    aFc_hi = static_cast<float*>(h->dev_buf("solve.altB.Fc_hi", nc * 4));
-    aFc_lo = static_cast<float*>(h->dev_buf("solve.altB.Fc_lo", nc * 4));
-    pongFr = static_cast<float*>(h->dev_buf("solve.pong.Fr", nr * 4));
-    if (!aFr || !aFr_hi || !aFr_lo || !aFc || !aFc_hi || !aFc_lo || !pongFr) return -2;
-  }
   CNMF_TRY(emit_pieces(0));        // f16: the callers' tf32 pieces are replaced by fp16 pieces of the initial factors
   CNMF_TRY(emit_pieces(1));
 
@@ -539,16 +451,9 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
     for (it = 1; it <= p.max_iter; ++it) {
       const bool check = (p.tol > 0 && it % 10 == 0) || it == p.max_iter;
       if (io.update_cols) {
-        if (fuse_w) {
-          CNMF_TRY(gemm_rows_fused(l1W, l2W));       // GEMM + update + pieces + Gram partials in one launch
-          std::swap(wFr, pongFr);
-          h->launches += 1;
-          CNMF_TRY(launch_finalize(d_gpartR, d_gramR, nullptr, nullptr, ntiles_r, bm(), s));
-        } else {
-          CNMF_TRY(gemm_rows());
-          CNMF_TRY(update(false, fr(), NUMr, plan_r, d_gramC, l1W, l2W, fused_out(0, true, nullptr, nullptr)));
-          CNMF_TRY(gram_after(fr(), 0));
-        }
+        CNMF_TRY(gemm_rows());
+        CNMF_TRY(update(false, fr(), NUMr, plan_r, d_gramC, l1W, l2W, fused_out(0, true, nullptr, nullptr)));
+        CNMF_TRY(gram_after(fr(), 0));
         CNMF_TRY(gemm_cols());
         CNMF_TRY(update(false, fc(), NUMc, plan_c, d_gramR, l1H, l2H, fused_out(1, true, check ? d_scalB : nullptr, d_crossB)));
         CNMF_TRY(gram_after(fc(), 1));

@@ -183,12 +183,12 @@ __global__ void sums_final_kernel(const double* __restrict__ part, int nblocks, 
 // The pieces are a pure function of the factor values: this stand-alone kernel (initial factors, re-packing after a
 // compaction, K > 16 batches) and the in-update emission (emit_tile_f16) produce the same bits, so a restart's
 // operands do not depend on when the batch around it was compacted.
-// One block per row, one warp per group of 128 * QUADS columns (512: what the update kernels' tiles emit; 128: what the
-// fused GEMM epilogue emits, one group per thread), a lane owns QUADS 16-byte quads of the group.
-template <int QUADS>
+// One block per row, one warp per group of 512 columns (what the update kernels' tiles emit), a lane owns QUADS = 4
+// 16-byte quads of the group.
 __global__ void __launch_bounds__(256)
 emit_f16_kernel(const float* __restrict__ F, int n, int ld, const float* __restrict__ pscale, __half* __restrict__ hi,
                 __half* __restrict__ mid, float* __restrict__ tile_scale, int n_ktiles) {
+  constexpr int QUADS = 4;
   const long long row = blockIdx.x;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const float* src = F + row * ld;
@@ -1301,16 +1301,11 @@ int launch_split_scaled(const float* src, float* hi, float* lo, int rows, int ld
 }
 
 int launch_emit_f16(const float* F, int rows, int n, int ld, const float* pscale, void* hi, void* mid, float* tile_scale,
-                    int n_ktiles, cudaStream_t s, int group) {
-  CNMF_REQUIRE(group == 512 || group == 128, "emit_f16: scale groups hold 512 or 128 elements");
-  CNMF_REQUIRE(ld % 8 == 0 && (long long)n_ktiles * group >= ld, "emit_f16: bad ld / n_ktiles");
+                    int n_ktiles, cudaStream_t s) {
+  CNMF_REQUIRE(ld % 8 == 0 && (long long)n_ktiles * 512 >= ld, "emit_f16: bad ld / n_ktiles");
   if (rows <= 0) return 0;
-  if (group == 512)
-    emit_f16_kernel<4><<<rows, 256, 0, s>>>(F, n, ld, pscale, static_cast<__half*>(hi), static_cast<__half*>(mid), tile_scale,
-                                            n_ktiles);
-  else
-    emit_f16_kernel<1><<<rows, 256, 0, s>>>(F, n, ld, pscale, static_cast<__half*>(hi), static_cast<__half*>(mid), tile_scale,
-                                            n_ktiles);
+  emit_f16_kernel<<<rows, 256, 0, s>>>(F, n, ld, pscale, static_cast<__half*>(hi), static_cast<__half*>(mid), tile_scale,
+                                       n_ktiles);
   CNMF_CUDA_CHECK(cudaGetLastError());
   return 0;
 }
@@ -1382,10 +1377,16 @@ int launch_matrix_sums(const float* X, int rows, int cols, int ld, double* out2,
     default: set_last_error("kp must be 16 or 32"); return -1;       \
   }
 
-template <int KPMAX, bool CD, bool GRAM, int MINB, bool STREAMN>
+// MU with the fused Gram at kp == 16 streams the products from global memory one component ahead of their use (no
+// product tile in shared memory) at 4 blocks per SM (128 registers); every other form stages what it needs in shared
+// memory at 3 (kp 16) or 2 (kp 32) blocks per SM.  The streamed form was the fastest of the layouts and occupancies
+// measured on c3 (profiles/r2m_update_variants.log); the kernel is bound by its instruction count, not by occupancy.
+template <int KPMAX, bool CD, bool GRAM>
 static int launch_update_inst(dim3 grid, const FactorView& f, const float* NUM, int nsplit, long long sstride,
                               const double* gram_in, const BatchMeta& b, float l1, float l2, const FusedOut& out,
                               cudaStream_t s) {
+  constexpr bool STREAMN = KPMAX == 16 && !CD && GRAM;
+  constexpr int MINB = STREAMN ? 4 : (KPMAX == 32 ? 2 : 3);
   // MU stages the thread's factor values (and, unless the products are streamed, the products) in shared memory
   // (rolled component loop); CD only needs the tile when it also emits the Gram
   const size_t smem = sizeof(float) * (CD ? (GRAM ? (size_t)UPD_TILE_F_FLOATS : 0)
@@ -1403,37 +1404,6 @@ static int launch_update_inst(dim3 grid, const FactorView& f, const float* NUM, 
   return 0;
 }
 
-// MU with the fused Gram at kp == 16, CNMF_UPD_VARIANT: 2 (default) = products streamed from global memory one
-// component ahead of their use, no product tile in shared memory, 4 blocks per SM (128 registers); 0 = round 1's
-// layout (products staged in a second shared-memory tile, 3 blocks per SM); 1 / 3 = streamed at 3 / 5 blocks per SM.
-// Measured on c3 (profiles/r2m_update_variants.log): update launches 1031 / 1085 / 962 / 1065 ms per 3 steps for
-// variants 0 / 1 / 2 / 3 -- the kernel is bound by its instruction count, not by occupancy; every variant computes the
-// same bits.
-static int upd_variant() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("CNMF_UPD_VARIANT");
-    v = e ? atoi(e) : 2;
-    if (v < 0 || v > 3) v = 2;
-  }
-  return v;
-}
-
-template <int KPMAX, bool CD, bool GRAM>
-static int launch_update_variant(dim3 grid, const FactorView& f, const float* NUM, int nsplit, long long sstride,
-                                 const double* gram_in, const BatchMeta& b, float l1, float l2, const FusedOut& out,
-                                 cudaStream_t s) {
-  if constexpr (KPMAX == 16 && !CD && GRAM) {
-    switch (upd_variant()) {
-      case 1: return launch_update_inst<KPMAX, CD, GRAM, 3, true>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
-      case 2: return launch_update_inst<KPMAX, CD, GRAM, 4, true>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
-      case 3: return launch_update_inst<KPMAX, CD, GRAM, 5, true>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
-      default: break;
-    }
-  }
-  return launch_update_inst<KPMAX, CD, GRAM, (KPMAX == 32 ? 2 : 3), false>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
-}
-
 template <bool CD>
 static int launch_update(const FactorView& f, const float* NUM, int nsplit, long long sstride, const double* gram_in,
                          const BatchMeta& b, float l1, float l2, const FusedOut& out, cudaStream_t s) {
@@ -1442,12 +1412,12 @@ static int launch_update(const FactorView& f, const float* NUM, int nsplit, long
   static_assert(16 * UPD_THREADS * 4 == UPD_TILE_N_FLOATS && 32 * UPD_THREADS * 2 == UPD_TILE_N_FLOATS, "tile sizes");
   dim3 grid(col_chunks(f), b.R);
   if (b.kp == 16) {
-    if (out.gram_part) return launch_update_variant<16, CD, true>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
-    return launch_update_variant<16, CD, false>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
+    if (out.gram_part) return launch_update_inst<16, CD, true>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
+    return launch_update_inst<16, CD, false>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
   }
   if (b.kp == 32) {
     CNMF_REQUIRE(out.gram_part == nullptr, "update: the fused Gram exists for kp == 16 batches only");
-    return launch_update_variant<32, CD, false>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
+    return launch_update_inst<32, CD, false>(grid, f, NUM, nsplit, sstride, gram_in, b, l1, l2, out, s);
   }
   set_last_error("kp must be 16 or 32");
   return -1;

@@ -64,11 +64,11 @@ int launch_split_tf32(const float* src, float* hi, float* lo, long long n_elems,
 int launch_split_scaled(const float* src, float* hi, float* lo, int rows, int ld, const float* col_scale, cudaStream_t s);
 
 // ---- fp16 operand pieces (f16x2 precision, exact-count datasets) ----
-// per packed row r and group g of `group` (512 or 128) columns: sc = power of two with max(F[r, c] * pscale[c]) / sc in
+// per packed row r and group g of 512 columns: sc = power of two with max(F[r, c] * pscale[c]) / sc in
 // [2^14, 2^15) over the group -> tile_scale[r * n_ktiles + g]; hi / mid (fp16, row stride ld halves) = the two pieces of
-// F[r, :] * pscale / sc.  Same bits as the in-kernel emissions (update kernels: groups of 512; fused GEMM epilogue: 128)
+// F[r, :] * pscale / sc.  Same bits as the update kernels' in-kernel emission
 int launch_emit_f16(const float* F, int rows, int n, int ld, const float* pscale, void* hi, void* mid, float* tile_scale,
-                    int n_ktiles, cudaStream_t s, int group = 512);
+                    int n_ktiles, cudaStream_t s);
 // dst (fp16) = src (fp32), elementwise; used for the exact integer count matrices
 int launch_to_half(const float* src, void* dst, long long n_elems, cudaStream_t s);
 

@@ -108,8 +108,8 @@ int cnmf_dataset_min(cnmf_dataset_t d, float* min_host, void* stream);
 /* 1 when the dataset was recognised as (row scale) x (integer counts <= 2048) x (column scale) -- what
  * HVG-normalised counts (cnmf.py:542) and TPM (cnmf.py:245-251) are -- and therefore runs the 2-pass
  * tensor-core products (the integer operand needs no tf32 "lo" piece); 0 = general 3-pass 3xTF32.
- * CNMF_EXACT=0 in the environment disables the detection.  Returns 2 when, in addition, the dataset was created with
- * CNMF_PRECISION_F16X2 and the 2 passes therefore run on kind::f16 MMAs. */
+ * Returns 2 when, in addition, the dataset was created with CNMF_PRECISION_F16X2 and the 2 passes therefore run on
+ * kind::f16 MMAs. */
 int cnmf_dataset_is_exact(cnmf_dataset_t d);
 /* per-column mean and population variance (StandardScaler(with_mean=False), cnmf.py:131-134) */
 int cnmf_dataset_col_stats(cnmf_dataset_t d, double* mean_host, double* var_host, void* stream);

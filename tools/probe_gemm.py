@@ -1,6 +1,5 @@
 #!/usr/bin/env python
-"""GPU probe: the batched GEMM alone on BASELINE-shaped problems (f16x2 path), mean device time per launch.
-CNMF_GEMM_PAIR=0/1 selects the 1-CTA / CTA-pair kernel (read once per process)."""
+"""GPU probe: the batched GEMM alone on BASELINE-shaped problems (f16x2 path), mean device time per launch."""
 import json, os, sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -9,7 +8,7 @@ from cnmf_b200.engine import Engine
 
 eng = Engine(0)
 rng = np.random.RandomState(0)
-out = {"pair": os.environ.get("CNMF_GEMM_PAIR", "1")}
+out = {}
 for name, (M, N, K, sp) in {"c2_W_half": (1000, 20000, 2000, 1), "c2_H_half": (1000, 2000, 20000, 5),
                             "mid_W_half": (4096, 16384, 2000, 1), "mid_H_half": (4096, 2000, 16384, 4),
                             "tail_H_half": (128, 2000, 20000, 5)}.items():
