@@ -27,12 +27,6 @@ void set_last_error(const std::string& msg) { g_last_error = msg; }
 
 using namespace cnmf;
 
-#define CNMF_TRY(expr)            \
-  do {                            \
-    int _rc = (expr);             \
-    if (_rc != 0) return _rc;     \
-  } while (0)
-
 // ----------------------------------------------------------------------------- handle
 void* cnmf_handle_s::dev_buf(const std::string& name, size_t bytes) {
   auto& e = ws[name];
@@ -171,13 +165,6 @@ int cnmf_create(cnmf_handle_t* out, int device) {
   auto* h = new cnmf_handle_s();
   h->device = device;
   h->sm_count = prop.multiProcessorCount;
-  {
-    int lo = 0, hi = 0;
-    cudaDeviceGetStreamPriorityRange(&lo, &hi);      // lo = lowest priority (numerically largest)
-    if (cudaStreamCreateWithPriority(&h->aux, cudaStreamNonBlocking, lo) != cudaSuccess) h->aux = nullptr;
-    if (cudaEventCreateWithFlags(&h->ev_upd, cudaEventDisableTiming) != cudaSuccess) h->ev_upd = nullptr;
-    if (cudaEventCreateWithFlags(&h->ev_gram, cudaEventDisableTiming) != cudaSuccess) h->ev_gram = nullptr;
-  }
   *out = h;
   return 0;
 }
@@ -185,9 +172,6 @@ int cnmf_create(cnmf_handle_t* out, int device) {
 int cnmf_destroy(cnmf_handle_t h) {
   if (!h) return 0;
   cudaSetDevice(h->device);
-  if (h->aux) cudaStreamDestroy(h->aux);
-  if (h->ev_upd) cudaEventDestroy(h->ev_upd);
-  if (h->ev_gram) cudaEventDestroy(h->ev_gram);
   h->release_all();
   delete h;
   return 0;
@@ -210,11 +194,12 @@ int cnmf_mem_info(cnmf_handle_t h, long long* free_bytes, long long* total_bytes
 
 long long cnmf_solve_bytes_per_row(cnmf_dataset_t d) {
   if (!d) return 0;
-  // nmf_engine.cu / alloc_factors: Fr + 2 piece buffers, their 3 compaction alternates, the result slab and the
-  // product NUM_r along the cells; the same along the genes with one product slice per split-K slice
+  // Floats per packed row along the cells (ld_r): the factor Fr and its 2 pieces (alloc_factors), their 3 compaction
+  // alternates and the result slab (solve_batched), one slice of the product NUM_r per split-K slice -- 7 + splits_r;
+  // along the genes (ld_c) the same for Fc -- 7 + splits_c.  The constants 11 and 10 count 4 and 3 rows more than
+  // that; the value stays as it is because callers size their restart groups from it.
   const long long splits_c = gemm_fixed_splits(d->n_rows, d->f16 ? 1 : 0);
   const long long splits_r = gemm_fixed_splits(d->n_cols, d->f16 ? 1 : 0);
-  // (+ the second ping-pong set and the output buffer of the fused W-half epilogue)
   return 4LL * ((11 + splits_r) * (long long)d->ld_r + (10 + splits_c) * (long long)d->ld_c);
 }
 
@@ -254,8 +239,12 @@ int cnmf_profile_get_class(cnmf_handle_t h, int cls, double* ms, long long* laun
   return 0;
 }
 
+}  // extern "C"
+
 // ----------------------------------------------------------------------------- dataset
-static int dataset_alloc(cnmf_dataset_s* d, float** p, size_t elems) {
+namespace cnmf {
+
+int dataset_alloc(cnmf_dataset_s* d, float** p, size_t elems) {
   const size_t bytes = std::max<size_t>(elems, 64) * sizeof(float);
   void* q = d->h->pool_take(bytes);
   if (!q) {
@@ -270,10 +259,7 @@ static int dataset_alloc(cnmf_dataset_s* d, float** p, size_t elems) {
   return 0;
 }
 
-int cnmf_dataset_alloc_internal(cnmf_dataset_t d, float** p, size_t elems) { return dataset_alloc(d, p, elems); }
-
-// builds Xt / tf32 pieces / sums from d->X (already resident, padding zeroed)
-static int dataset_finish(cnmf_dataset_s* d, cudaStream_t s) {
+int dataset_finish(cnmf_dataset_s* d, cudaStream_t s) {
   cnmf_handle_s* h = d->h;
   const size_t nx = (size_t)d->n_rows * d->ld_c, nxt = (size_t)d->n_cols * d->ld_r;
   if (d->precision == CNMF_PRECISION_TF32X3) {
@@ -323,15 +309,15 @@ static int dataset_finish(cnmf_dataset_s* d, cudaStream_t s) {
         d->drop_tf32 = true;
       }
     } else {
-    CNMF_TRY(dataset_alloc(d, &d->X_hi, nx));
-    CNMF_TRY(dataset_alloc(d, &d->X_lo, nx));
-    CNMF_TRY(dataset_alloc(d, &d->Xt_hi, nxt));
-    CNMF_TRY(dataset_alloc(d, &d->Xt_lo, nxt));
-    CNMF_CUDA_CHECK(cudaMemsetAsync(d->Xt_hi, 0, nxt * sizeof(float), s));
-    CNMF_CUDA_CHECK(cudaMemsetAsync(d->Xt_lo, 0, nxt * sizeof(float), s));
-    CNMF_TRY(launch_split_tf32(d->X, d->X_hi, d->X_lo, (long long)nx, s));
-    CNMF_TRY(launch_transpose(d->X, d->n_rows, d->n_cols, d->ld_c, nullptr, d->Xt_hi, d->Xt_lo, d->ld_r, s));
-    h->launches += 2;
+      CNMF_TRY(dataset_alloc(d, &d->X_hi, nx));
+      CNMF_TRY(dataset_alloc(d, &d->X_lo, nx));
+      CNMF_TRY(dataset_alloc(d, &d->Xt_hi, nxt));
+      CNMF_TRY(dataset_alloc(d, &d->Xt_lo, nxt));
+      CNMF_CUDA_CHECK(cudaMemsetAsync(d->Xt_hi, 0, nxt * sizeof(float), s));
+      CNMF_CUDA_CHECK(cudaMemsetAsync(d->Xt_lo, 0, nxt * sizeof(float), s));
+      CNMF_TRY(launch_split_tf32(d->X, d->X_hi, d->X_lo, (long long)nx, s));
+      CNMF_TRY(launch_transpose(d->X, d->n_rows, d->n_cols, d->ld_c, nullptr, d->Xt_hi, d->Xt_lo, d->ld_r, s));
+      h->launches += 2;
     }
   } else {
     CNMF_TRY(dataset_alloc(d, &d->Xt, nxt));
@@ -364,37 +350,28 @@ static int dataset_finish(cnmf_dataset_s* d, cudaStream_t s) {
   return 0;
 }
 
-int cnmf_dataset_create(cnmf_handle_t h, const float* X, int n_rows, int n_cols, long long ld, int src_is_device,
-                        int precision, void* stream, cnmf_dataset_t* out) {
-  CNMF_REQUIRE(h && X && out, "dataset_create: NULL argument");
-  CNMF_REQUIRE(n_rows > 0 && n_cols > 0 && ld >= n_cols, "dataset_create: bad shape");
-  CNMF_REQUIRE(precision == CNMF_PRECISION_FP32 || precision == CNMF_PRECISION_TF32X3 ||
-                   precision == CNMF_PRECISION_TF32X3_GENERAL || precision == CNMF_PRECISION_F16X2,
-               "dataset_create: bad precision");
-  cudaStream_t s = as_stream(stream);
-  CNMF_CUDA_CHECK(cudaSetDevice(h->device));
+int dataset_new(cnmf_handle_s* h, const cnmf_dataset_s* like, int precision, int n_rows, int n_cols,
+                cnmf_dataset_s** out) {
   auto* d = new cnmf_dataset_s();
   d->h = h;
   d->n_rows = n_rows;
   d->n_cols = n_cols;
   d->ld_c = pad_ld(n_cols);
   d->ld_r = pad_ld(n_rows);
-  d->allow_exact = precision != CNMF_PRECISION_TF32X3_GENERAL;
-  d->want_f16 = precision == CNMF_PRECISION_F16X2;
-  d->precision = (precision == CNMF_PRECISION_TF32X3_GENERAL || precision == CNMF_PRECISION_F16X2) ? CNMF_PRECISION_TF32X3
-                                                                                                : precision;
-  int rc = dataset_alloc(d, &d->X, (size_t)n_rows * d->ld_c);
-  if (rc == 0) {
-    cudaError_t e = cudaMemsetAsync(d->X, 0, (size_t)n_rows * d->ld_c * sizeof(float), s);
-    if (e == cudaSuccess)
-      e = cudaMemcpy2DAsync(d->X, (size_t)d->ld_c * sizeof(float), X, (size_t)ld * sizeof(float),
-                            (size_t)n_cols * sizeof(float), n_rows,
-                            src_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) {
-      set_last_error(std::string("dataset upload failed: ") + cudaGetErrorString(e));
-      rc = -2;
-    }
+  d->allow_exact = like ? like->allow_exact : precision != CNMF_PRECISION_TF32X3_GENERAL;
+  d->want_f16 = like ? like->want_f16 : precision == CNMF_PRECISION_F16X2;
+  // GENERAL and F16X2 are TF32X3 datasets that differ in these two flags
+  d->precision = like ? like->precision : (d->allow_exact && !d->want_f16 ? precision : CNMF_PRECISION_TF32X3);
+  const int rc = dataset_alloc(d, &d->X, (size_t)n_rows * d->ld_c);
+  if (rc != 0) {
+    cnmf_dataset_destroy(d);
+    return rc;
   }
+  *out = d;
+  return 0;
+}
+
+int finish_or_destroy(cnmf_dataset_s* d, int rc, cudaStream_t s, cnmf_dataset_t* out) {
   if (rc == 0) rc = dataset_finish(d, s);
   if (rc != 0) {
     cnmf_dataset_destroy(d);
@@ -404,7 +381,270 @@ int cnmf_dataset_create(cnmf_handle_t h, const float* X, int n_rows, int n_cols,
   return 0;
 }
 
-int cnmf_dataset_finish_internal(cnmf_dataset_t d, void* stream) { return dataset_finish(d, as_stream(stream)); }
+int dataset_ensure_full_transpose(cnmf_dataset_s* d, cudaStream_t s) {
+  if (d->Xt) return 0;
+  CNMF_CUDA_CHECK(cudaSetDevice(d->h->device));
+  const size_t nxt = (size_t)d->n_cols * d->ld_r;
+  CNMF_TRY(dataset_alloc(d, &d->Xt, nxt));
+  CNMF_CUDA_CHECK(cudaMemsetAsync(d->Xt, 0, nxt * sizeof(float), s));
+  CNMF_TRY(launch_transpose(d->X, d->n_rows, d->n_cols, d->ld_c, d->Xt, nullptr, nullptr, d->ld_r, s));
+  d->h->launches += 1;
+  CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+// ----------------------------------------------------------------------------- factorize
+int alloc_factors(cnmf_handle_s* h, const char* prefix, int SK, int ld_r, int ld_c, bool tf32, SolveIO* io) {
+  const std::string pre(prefix);
+  const size_t nr = (size_t)SK * ld_r, nc = (size_t)SK * ld_c;
+  io->Fr = static_cast<float*>(h->dev_buf(pre + "Fr", nr * 4));
+  io->Fc = static_cast<float*>(h->dev_buf(pre + "Fc", nc * 4));
+  if (!io->Fr || !io->Fc) return -2;
+  if (tf32) {
+    io->Fr_hi = static_cast<float*>(h->dev_buf(pre + "Fr_hi", nr * 4));
+    io->Fr_lo = static_cast<float*>(h->dev_buf(pre + "Fr_lo", nr * 4));
+    io->Fc_hi = static_cast<float*>(h->dev_buf(pre + "Fc_hi", nc * 4));
+    io->Fc_lo = static_cast<float*>(h->dev_buf(pre + "Fc_lo", nc * 4));
+    if (!io->Fr_hi || !io->Fr_lo || !io->Fc_hi || !io->Fc_lo) return -2;
+  }
+  return 0;
+}
+
+int split_factors(cnmf_handle_s* h, const DataView& v, const SolveIO& io, int SK, bool tf32, cudaStream_t s) {
+  if (!tf32 || v.f16) return 0;
+  CNMF_TRY(launch_split_scaled(io.Fr, io.Fr_hi, io.Fr_lo, SK, v.ld_r, v.exact ? v.scale_r : nullptr, s));
+  CNMF_TRY(launch_split_scaled(io.Fc, io.Fc_hi, io.Fc_lo, SK, v.ld_c, v.exact ? v.scale_c : nullptr, s));
+  h->launches += 2;
+  return 0;
+}
+
+}  // namespace cnmf
+
+namespace {
+
+using clk = std::chrono::steady_clock;
+double ms_since(clk::time_point t0) { return std::chrono::duration<double, std::milli>(clk::now() - t0).count(); }
+
+// The restarts of one call: K of each, their packed row offsets, the total rows SK and the scale of sklearn's random
+// init, sqrt(mean(X) / k)
+struct RestartTable {
+  std::vector<int> ks, off;
+  std::vector<double> avgs;
+  int SK = 0;
+};
+
+int restart_table(const cnmf_dataset_s* d, int n_restarts, const int32_t* ks_in, RestartTable* t) {
+  const double mean = d->sum / ((double)d->n_rows * (double)d->n_cols);
+  t->ks.assign(ks_in, ks_in + n_restarts);
+  t->off.resize(n_restarts);
+  t->avgs.resize(n_restarts);
+  for (int r = 0; r < n_restarts; ++r) {
+    CNMF_REQUIRE(t->ks[r] >= 1 && t->ks[r] <= KMAX, "n_components must be in [1, 32] on the CUDA path");
+    t->off[r] = t->SK;
+    t->SK += t->ks[r];
+    t->avgs[r] = std::sqrt(mean / t->ks[r]);
+  }
+  return 0;
+}
+
+// the legacy MT19937 / polar-gauss stream of every restart, generated in place on the GPU into packed padded factors
+int device_rng(cnmf_dataset_s* d, const RestartTable& t, const uint32_t* seeds, float* Fr, float* Fc, cudaStream_t s) {
+  CNMF_CUDA_CHECK(cudaMemsetAsync(Fr, 0, (size_t)t.SK * d->ld_r * 4, s));
+  CNMF_CUDA_CHECK(cudaMemsetAsync(Fc, 0, (size_t)t.SK * d->ld_c * 4, s));
+  return launch_rng_init(seeds, t.ks.data(), t.off.data(), t.avgs.data(), (int)t.ks.size(), d->n_rows, d->n_cols, Fr,
+                         d->ld_r, Fc, d->ld_c, d->h, s);
+}
+
+void parallel_for(int n, const std::function<void(int)>& fn) {
+  int nt = (int)std::thread::hardware_concurrency();
+  if (nt < 1) nt = 1;
+  nt = std::min(nt, n);
+  if (nt <= 1) {
+    for (int i = 0; i < n; ++i) fn(i);
+    return;
+  }
+  std::atomic<int> next{0};
+  std::vector<std::thread> th;
+  th.reserve(nt);
+  for (int t = 0; t < nt; ++t)
+    th.emplace_back([&] {
+      for (;;) {
+        const int i = next.fetch_add(1);
+        if (i >= n) break;
+        fn(i);
+      }
+    });
+  for (auto& t : th) t.join();
+}
+
+// the same stream on the host (bit-exact numpy), in groups through a pinned staging buffer
+int host_rng(cnmf_dataset_s* d, const RestartTable& t, const uint32_t* seeds, float* Fr, float* Fc, cudaStream_t s) {
+  cnmf_handle_s* h = d->h;
+  const std::vector<int>& ks = t.ks;
+  const std::vector<int>& off = t.off;
+  const int n_restarts = (int)ks.size();
+  const size_t group_budget = (size_t)256 << 20;   // bytes of W^T staged per group
+  int r0 = 0;
+  while (r0 < n_restarts) {
+    int r1 = r0;
+    size_t bytes = 0;
+    while (r1 < n_restarts && (r1 == r0 || bytes + (size_t)ks[r1] * d->ld_r * 4 <= group_budget)) {
+      bytes += (size_t)ks[r1] * d->ld_r * 4;
+      ++r1;
+    }
+    const int rows = off[r1 - 1] + ks[r1 - 1] - off[r0];
+    float* stW = static_cast<float*>(h->host_buf("stage.W", (size_t)rows * d->ld_r * 4));
+    float* stH = static_cast<float*>(h->host_buf("stage.H", (size_t)rows * d->ld_c * 4));
+    if (!stW || !stH) return -2;
+    auto t_rng = clk::now();
+    parallel_for(r1 - r0, [&](int i) {
+      const int r = r0 + i;
+      float* w = stW + (size_t)(off[r] - off[r0]) * d->ld_r;
+      float* hh = stH + (size_t)(off[r] - off[r0]) * d->ld_c;
+      nmf_random_init(seeds[r], t.avgs[r], d->n_rows, d->n_cols, ks[r], w, d->ld_r, hh, d->ld_c);
+      for (int c = 0; c < ks[r]; ++c) {                  // zero the row padding (each worker its own rows)
+        std::memset(w + (size_t)c * d->ld_r + d->n_rows, 0, (size_t)(d->ld_r - d->n_rows) * 4);
+        std::memset(hh + (size_t)c * d->ld_c + d->n_cols, 0, (size_t)(d->ld_c - d->n_cols) * 4);
+      }
+    });
+    h->t_rng_ms += ms_since(t_rng);
+    auto t_h2d = clk::now();
+    CNMF_CUDA_CHECK(cudaMemcpyAsync(Fr + (size_t)off[r0] * d->ld_r, stW, (size_t)rows * d->ld_r * 4,
+                                    cudaMemcpyHostToDevice, s));
+    CNMF_CUDA_CHECK(cudaMemcpyAsync(Fc + (size_t)off[r0] * d->ld_c, stH, (size_t)rows * d->ld_c * 4,
+                                    cudaMemcpyHostToDevice, s));
+    CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
+    h->t_h2d_ms += ms_since(t_h2d);
+    r0 = r1;
+  }
+  return 0;
+}
+
+// Where the starting factors of a factorize come from: the seeded generator on the device or on the host, or packed
+// factors of the caller (host: rows of n_rows / n_cols floats; device: rows padded to the dataset's ld)
+struct Starts {
+  enum Kind { DEVICE_RNG, HOST_RNG, HOST_FACTORS, DEVICE_FACTORS } kind;
+  const uint32_t* seeds;
+  const float* Wt0;
+  const float* H0;
+};
+
+Starts seeded(const cnmf_nmf_params& p, const uint32_t* seeds) {
+  return {(p.reserved & 1) ? Starts::HOST_RNG : Starts::DEVICE_RNG, seeds, nullptr, nullptr};
+}
+
+// Where the results go: spectra (and usages, if set) to the host as packed rows of n_cols (n_rows) floats, or spectra
+// to the device as the first `width` floats of rows `ld` apart; per-restart statistics to the host
+struct Outputs {
+  float* spectra_host;
+  float* usages_host;
+  float* spectra_dev;
+  long long ld, width;
+  int32_t* n_iter_host;
+  double* err_host;
+};
+
+// The one host path of every factorize entry point: starting factors into the "fac." workspace, tf32 pieces, the
+// batched solve, results out.  Resets and fills the handle's phase timings.
+int factorize_run(cnmf_dataset_s* d, int n_restarts, const int32_t* ks_in, const cnmf_nmf_params& p, const Starts& in,
+                  const Outputs& out, void* stream) {
+  cnmf_handle_s* h = d->h;
+  cudaStream_t s = as_stream(stream);
+  CNMF_CUDA_CHECK(cudaSetDevice(h->device));
+  RestartTable t;
+  CNMF_TRY(restart_table(d, n_restarts, ks_in, &t));
+  const int SK = t.SK;
+  const bool tf32 = p.precision == CNMF_PRECISION_TF32X3;
+  SolveIO io;
+  CNMF_TRY(alloc_factors(h, "fac.", SK, d->ld_r, d->ld_c, tf32, &io));
+  h->t_rng_ms = h->t_h2d_ms = h->t_solve_ms = h->t_d2h_ms = 0;
+  switch (in.kind) {
+    case Starts::DEVICE_RNG: {
+      // no host synchronisation: launch_rng_init stages its arguments itself, and the solve is enqueued behind the
+      // generator on the same stream (t_rng_ms = enqueue time; the kernel's time is part of t_solve_ms)
+      const auto t_rng = clk::now();
+      CNMF_TRY(device_rng(d, t, in.seeds, io.Fr, io.Fc, s));
+      h->t_rng_ms = ms_since(t_rng);
+      break;
+    }
+    case Starts::HOST_RNG:
+      CNMF_TRY(host_rng(d, t, in.seeds, io.Fr, io.Fc, s));
+      break;
+    case Starts::HOST_FACTORS:
+      CNMF_CUDA_CHECK(cudaMemsetAsync(io.Fr, 0, (size_t)SK * d->ld_r * 4, s));
+      CNMF_CUDA_CHECK(cudaMemsetAsync(io.Fc, 0, (size_t)SK * d->ld_c * 4, s));
+      CNMF_CUDA_CHECK(cudaMemcpy2DAsync(io.Fr, (size_t)d->ld_r * 4, in.Wt0, (size_t)d->n_rows * 4,
+                                        (size_t)d->n_rows * 4, SK, cudaMemcpyHostToDevice, s));
+      CNMF_CUDA_CHECK(cudaMemcpy2DAsync(io.Fc, (size_t)d->ld_c * 4, in.H0, (size_t)d->n_cols * 4,
+                                        (size_t)d->n_cols * 4, SK, cudaMemcpyHostToDevice, s));
+      break;
+    case Starts::DEVICE_FACTORS:
+      CNMF_CUDA_CHECK(cudaMemcpyAsync(io.Fr, in.Wt0, (size_t)SK * d->ld_r * 4, cudaMemcpyDeviceToDevice, s));
+      CNMF_CUDA_CHECK(cudaMemcpyAsync(io.Fc, in.H0, (size_t)SK * d->ld_c * 4, cudaMemcpyDeviceToDevice, s));
+      break;
+  }
+  const DataView v = make_view(d, false);
+  CNMF_TRY(split_factors(h, v, io, SK, tf32, s));
+  io.R = n_restarts;
+  io.ks = t.ks;
+  io.update_cols = true;
+  const auto t_solve = clk::now();
+  CNMF_TRY(solve_batched(h, v, io, p, s));
+  h->t_solve_ms = ms_since(t_solve);
+  const auto t_d2h = clk::now();
+  if (out.spectra_dev)
+    CNMF_CUDA_CHECK(cudaMemcpy2DAsync(out.spectra_dev, (size_t)out.ld * 4, io.Fc, (size_t)d->ld_c * 4,
+                                      (size_t)out.width * 4, SK, cudaMemcpyDeviceToDevice, s));
+  if (out.spectra_host)
+    CNMF_CUDA_CHECK(cudaMemcpy2DAsync(out.spectra_host, (size_t)d->n_cols * 4, io.Fc, (size_t)d->ld_c * 4,
+                                      (size_t)d->n_cols * 4, SK, cudaMemcpyDeviceToHost, s));
+  if (out.usages_host)
+    CNMF_CUDA_CHECK(cudaMemcpy2DAsync(out.usages_host, (size_t)d->n_rows * 4, io.Fr, (size_t)d->ld_r * 4,
+                                      (size_t)d->n_rows * 4, SK, cudaMemcpyDeviceToHost, s));
+  CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
+  h->t_d2h_ms = ms_since(t_d2h);
+  for (int r = 0; r < n_restarts; ++r) {
+    if (out.n_iter_host) out.n_iter_host[r] = io.n_iter[r];
+    if (out.err_host) out.err_host[r] = io.err[r];
+  }
+  return 0;
+}
+
+int check_params(cnmf_dataset_s* d, const cnmf_nmf_params* p) {
+  CNMF_REQUIRE(d && p, "NULL dataset or params");
+  CNMF_REQUIRE(p->precision == d->precision, "params.precision must match the precision the dataset was created with");
+  CNMF_REQUIRE(p->reserved2 == 0, "params.reserved2 must be 0");
+  if (p->beta_loss != CNMF_LOSS_FROBENIUS) CNMF_TRY(cnmf::dataset_ensure_full_transpose(d, nullptr));
+  return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int cnmf_dataset_create(cnmf_handle_t h, const float* X, int n_rows, int n_cols, long long ld, int src_is_device,
+                        int precision, void* stream, cnmf_dataset_t* out) {
+  CNMF_REQUIRE(h && X && out, "dataset_create: NULL argument");
+  CNMF_REQUIRE(n_rows > 0 && n_cols > 0 && ld >= n_cols, "dataset_create: bad shape");
+  CNMF_REQUIRE(precision == CNMF_PRECISION_FP32 || precision == CNMF_PRECISION_TF32X3 ||
+                   precision == CNMF_PRECISION_TF32X3_GENERAL || precision == CNMF_PRECISION_F16X2,
+               "dataset_create: bad precision");
+  cudaStream_t s = as_stream(stream);
+  CNMF_CUDA_CHECK(cudaSetDevice(h->device));
+  cnmf_dataset_s* d = nullptr;
+  CNMF_TRY(dataset_new(h, nullptr, precision, n_rows, n_cols, &d));
+  int rc = 0;
+  cudaError_t e = cudaMemsetAsync(d->X, 0, (size_t)n_rows * d->ld_c * sizeof(float), s);
+  if (e == cudaSuccess)
+    e = cudaMemcpy2DAsync(d->X, (size_t)d->ld_c * sizeof(float), X, (size_t)ld * sizeof(float),
+                          (size_t)n_cols * sizeof(float), n_rows,
+                          src_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, s);
+  if (e != cudaSuccess) {
+    set_last_error(std::string("dataset upload failed: ") + cudaGetErrorString(e));
+    rc = -2;
+  }
+  return finish_or_destroy(d, rc, s, out);
+}
 
 int cnmf_dataset_min(cnmf_dataset_t d, float* min_host, void* stream) {
   CNMF_REQUIRE(d && min_host, "dataset_min: NULL argument");
@@ -444,190 +684,25 @@ int cnmf_random_init_host(uint32_t seed, double avg, int n_samples, int n_featur
   return 0;
 }
 
-// ----------------------------------------------------------------------------- factorize
-namespace {
-
-struct FactorBuffers {
-  float *Fr, *Fr_hi, *Fr_lo, *Fc, *Fc_hi, *Fc_lo;
-};
-
-int alloc_factors(cnmf_handle_s* h, int SK, int ld_r, int ld_c, bool tf32, FactorBuffers* fb) {
-  const size_t nr = (size_t)SK * ld_r, nc = (size_t)SK * ld_c;
-  fb->Fr = static_cast<float*>(h->dev_buf("fac.Fr", nr * 4));
-  fb->Fc = static_cast<float*>(h->dev_buf("fac.Fc", nc * 4));
-  fb->Fr_hi = fb->Fr_lo = fb->Fc_hi = fb->Fc_lo = nullptr;
-  if (!fb->Fr || !fb->Fc) return -2;
-  if (tf32) {
-    fb->Fr_hi = static_cast<float*>(h->dev_buf("fac.Fr_hi", nr * 4));
-    fb->Fr_lo = static_cast<float*>(h->dev_buf("fac.Fr_lo", nr * 4));
-    fb->Fc_hi = static_cast<float*>(h->dev_buf("fac.Fc_hi", nc * 4));
-    fb->Fc_lo = static_cast<float*>(h->dev_buf("fac.Fc_lo", nc * 4));
-    if (!fb->Fr_hi || !fb->Fr_lo || !fb->Fc_hi || !fb->Fc_lo) return -2;
-  }
-  return 0;
-}
-
-void parallel_for(int n, const std::function<void(int)>& fn) {
-  int nt = (int)std::thread::hardware_concurrency();
-  if (nt < 1) nt = 1;
-  nt = std::min(nt, n);
-  if (nt <= 1) {
-    for (int i = 0; i < n; ++i) fn(i);
-    return;
-  }
-  std::atomic<int> next{0};
-  std::vector<std::thread> th;
-  th.reserve(nt);
-  for (int t = 0; t < nt; ++t)
-    th.emplace_back([&] {
-      for (;;) {
-        const int i = next.fetch_add(1);
-        if (i >= n) break;
-        fn(i);
-      }
-    });
-  for (auto& t : th) t.join();
-}
-
-// shared tail of cnmf_factorize / cnmf_factorize_init: factors already in fb.Fr / fb.Fc (full fp32)
-int run_and_download(cnmf_dataset_s* d, const std::vector<int>& ks, int SK, FactorBuffers& fb,
-                     const cnmf_nmf_params& p, float* spectra_host, float* usages_host, int32_t* n_iter_host,
-                     double* err_host, cudaStream_t s, float* spectra_dev = nullptr, long long ld_dev = 0) {
-  cnmf_handle_s* h = d->h;
-  const bool tf32 = p.precision == CNMF_PRECISION_TF32X3;
-  DataView v = make_view(d, false);
-  if (tf32 && !v.f16) {      // f16 datasets: the solver emits fp16 pieces itself; tf32 pieces would be dead work
-    CNMF_TRY(launch_split_scaled(fb.Fr, fb.Fr_hi, fb.Fr_lo, SK, d->ld_r, v.exact ? v.scale_r : nullptr, s));
-    CNMF_TRY(launch_split_scaled(fb.Fc, fb.Fc_hi, fb.Fc_lo, SK, d->ld_c, v.exact ? v.scale_c : nullptr, s));
-    h->launches += 2;
-  }
-  SolveIO io;
-  io.R = (int)ks.size();
-  io.ks = ks;
-  io.Fr = fb.Fr; io.Fr_hi = fb.Fr_hi; io.Fr_lo = fb.Fr_lo;
-  io.Fc = fb.Fc; io.Fc_hi = fb.Fc_hi; io.Fc_lo = fb.Fc_lo;
-  io.update_cols = true;
-  auto t_solve = std::chrono::steady_clock::now();
-  CNMF_TRY(solve_batched(h, v, io, p, s));
-  h->t_solve_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_solve).count();
-  auto t_d2h = std::chrono::steady_clock::now();
-  if (spectra_dev)      // result stays in HBM (multi-GPU path: the slab goes straight into the NCCL all-gather)
-    CNMF_CUDA_CHECK(cudaMemcpy2DAsync(spectra_dev, (size_t)ld_dev * 4, fb.Fc, (size_t)d->ld_c * 4,
-                                      (size_t)d->n_cols * 4, SK, cudaMemcpyDeviceToDevice, s));
-  if (spectra_host)
-    CNMF_CUDA_CHECK(cudaMemcpy2DAsync(spectra_host, (size_t)d->n_cols * 4, fb.Fc, (size_t)d->ld_c * 4,
-                                      (size_t)d->n_cols * 4, SK, cudaMemcpyDeviceToHost, s));
-  if (usages_host)
-    CNMF_CUDA_CHECK(cudaMemcpy2DAsync(usages_host, (size_t)d->n_rows * 4, fb.Fr, (size_t)d->ld_r * 4,
-                                      (size_t)d->n_rows * 4, SK, cudaMemcpyDeviceToHost, s));
-  CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
-  h->t_d2h_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_d2h).count();
-  for (size_t r = 0; r < ks.size(); ++r) {
-    if (n_iter_host) n_iter_host[r] = io.n_iter[r];
-    if (err_host) err_host[r] = io.err[r];
-  }
-  return 0;
-}
-
-int check_params(cnmf_dataset_s* d, const cnmf_nmf_params* p) {
-  CNMF_REQUIRE(d && p, "NULL dataset or params");
-  CNMF_REQUIRE(p->precision == d->precision, "params.precision must match the precision the dataset was created with");
-  CNMF_REQUIRE(p->reserved2 == 0, "params.reserved2 must be 0");
-  if (p->beta_loss != CNMF_LOSS_FROBENIUS) CNMF_TRY(cnmf::dataset_ensure_full_transpose(d, nullptr));
-  return 0;
-}
-
-}  // namespace
-
-static int factorize_impl(cnmf_dataset_t d, int n_restarts, const int32_t* ks_in, const uint32_t* seeds,
-                          const cnmf_nmf_params* p, float* spectra_host, float* usages_host, int32_t* n_iter_host,
-                          double* err_host, void* stream, float* spectra_dev, long long ld_dev) {
-  CNMF_TRY(check_params(d, p));
-  CNMF_REQUIRE(n_restarts > 0 && ks_in && seeds && (spectra_host || spectra_dev), "factorize: bad arguments");
-  CNMF_REQUIRE(!spectra_dev || ld_dev >= d->n_cols, "factorize: device output row stride too small");
-  cnmf_handle_s* h = d->h;
-  cudaStream_t s = as_stream(stream);
-  CNMF_CUDA_CHECK(cudaSetDevice(h->device));
-  std::vector<int> ks(ks_in, ks_in + n_restarts), off(n_restarts);
-  int SK = 0;
-  for (int r = 0; r < n_restarts; ++r) {
-    CNMF_REQUIRE(ks[r] >= 1 && ks[r] <= KMAX, "factorize: n_components must be in [1, 32] on the CUDA path");
-    off[r] = SK;
-    SK += ks[r];
-  }
-  FactorBuffers fb;
-  CNMF_TRY(alloc_factors(h, SK, d->ld_r, d->ld_c, p->precision == CNMF_PRECISION_TF32X3, &fb));
-
-  using clk = std::chrono::steady_clock;
-  auto ms_since = [](clk::time_point t0) { return std::chrono::duration<double, std::milli>(clk::now() - t0).count(); };
-  h->t_rng_ms = h->t_h2d_ms = h->t_solve_ms = h->t_d2h_ms = 0;
-  if ((p->reserved & 1) == 0) {
-    // ---- device RNG (default): the same legacy MT19937 / polar-gauss stream, generated in place on the GPU
-    auto t_rng = clk::now();
-    const double mean_d = d->sum / ((double)d->n_rows * (double)d->n_cols);
-    std::vector<double> avgs(n_restarts);
-    for (int r = 0; r < n_restarts; ++r) avgs[r] = std::sqrt(mean_d / ks[r]);
-    CNMF_CUDA_CHECK(cudaMemsetAsync(fb.Fr, 0, (size_t)SK * d->ld_r * 4, s));
-    CNMF_CUDA_CHECK(cudaMemsetAsync(fb.Fc, 0, (size_t)SK * d->ld_c * 4, s));
-    CNMF_TRY(launch_rng_init(seeds, ks.data(), off.data(), avgs.data(), n_restarts, d->n_rows, d->n_cols, fb.Fr, d->ld_r,
-                             fb.Fc, d->ld_c, h, s));
-    // no host synchronisation here: launch_rng_init stages its arguments itself, and the solve is enqueued behind
-    // the generator on the same stream (t_rng_ms = enqueue time; the kernel's time is part of t_solve_ms)
-    h->t_rng_ms = ms_since(t_rng);
-    return run_and_download(d, ks, SK, fb, *p, spectra_host, usages_host, n_iter_host, err_host, s, spectra_dev, ld_dev);
-  }
-  // host RNG (bit-exact numpy legacy stream) in groups through a pinned staging buffer
-  const double mean = d->sum / ((double)d->n_rows * (double)d->n_cols);
-  const size_t group_budget = (size_t)256 << 20;   // bytes of W^T staged per group
-  int r0 = 0;
-  while (r0 < n_restarts) {
-    int r1 = r0;
-    size_t bytes = 0;
-    while (r1 < n_restarts && (r1 == r0 || bytes + (size_t)ks[r1] * d->ld_r * 4 <= group_budget)) {
-      bytes += (size_t)ks[r1] * d->ld_r * 4;
-      ++r1;
-    }
-    const int rows = off[r1 - 1] + ks[r1 - 1] - off[r0];
-    float* stW = static_cast<float*>(h->host_buf("stage.W", (size_t)rows * d->ld_r * 4));
-    float* stH = static_cast<float*>(h->host_buf("stage.H", (size_t)rows * d->ld_c * 4));
-    if (!stW || !stH) return -2;
-    auto t_rng = clk::now();
-    parallel_for(r1 - r0, [&](int i) {
-      const int r = r0 + i;
-      const double avg = std::sqrt(mean / ks[r]);
-      float* w = stW + (size_t)(off[r] - off[r0]) * d->ld_r;
-      float* hh = stH + (size_t)(off[r] - off[r0]) * d->ld_c;
-      nmf_random_init(seeds[r], avg, d->n_rows, d->n_cols, ks[r], w, d->ld_r, hh, d->ld_c);
-      for (int c = 0; c < ks[r]; ++c) {                  // zero the row padding (each worker its own rows)
-        std::memset(w + (size_t)c * d->ld_r + d->n_rows, 0, (size_t)(d->ld_r - d->n_rows) * 4);
-        std::memset(hh + (size_t)c * d->ld_c + d->n_cols, 0, (size_t)(d->ld_c - d->n_cols) * 4);
-      }
-    });
-    h->t_rng_ms += ms_since(t_rng);
-    auto t_h2d = clk::now();
-    CNMF_CUDA_CHECK(cudaMemcpyAsync(fb.Fr + (size_t)off[r0] * d->ld_r, stW, (size_t)rows * d->ld_r * 4,
-                                    cudaMemcpyHostToDevice, s));
-    CNMF_CUDA_CHECK(cudaMemcpyAsync(fb.Fc + (size_t)off[r0] * d->ld_c, stH, (size_t)rows * d->ld_c * 4,
-                                    cudaMemcpyHostToDevice, s));
-    CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
-    h->t_h2d_ms += ms_since(t_h2d);
-    r0 = r1;
-  }
-  return run_and_download(d, ks, SK, fb, *p, spectra_host, usages_host, n_iter_host, err_host, s, spectra_dev, ld_dev);
-}
-
 int cnmf_factorize(cnmf_dataset_t d, int n_restarts, const int32_t* ks_in, const uint32_t* seeds,
                    const cnmf_nmf_params* p, float* spectra_host, float* usages_host, int32_t* n_iter_host,
                    double* err_host, void* stream) {
   CNMF_REQUIRE(spectra_host, "factorize: spectra_host is NULL");
-  return factorize_impl(d, n_restarts, ks_in, seeds, p, spectra_host, usages_host, n_iter_host, err_host, stream, nullptr, 0);
+  CNMF_TRY(check_params(d, p));
+  CNMF_REQUIRE(n_restarts > 0 && ks_in && seeds, "factorize: bad arguments");
+  return factorize_run(d, n_restarts, ks_in, *p, seeded(*p, seeds),
+                       {spectra_host, usages_host, nullptr, 0, 0, n_iter_host, err_host}, stream);
 }
 
 int cnmf_factorize_seeds_dev(cnmf_dataset_t d, int n_restarts, const int32_t* ks_in, const uint32_t* seeds,
                              const cnmf_nmf_params* p, float* spectra_dev, long long ld_out, int32_t* n_iter_host,
                              double* err_host, void* stream) {
   CNMF_REQUIRE(spectra_dev, "factorize_seeds_dev: spectra_dev is NULL");
-  return factorize_impl(d, n_restarts, ks_in, seeds, p, nullptr, nullptr, n_iter_host, err_host, stream, spectra_dev, ld_out);
+  CNMF_TRY(check_params(d, p));
+  CNMF_REQUIRE(n_restarts > 0 && ks_in && seeds, "factorize: bad arguments");
+  CNMF_REQUIRE(ld_out >= d->n_cols, "factorize: device output row stride too small");
+  return factorize_run(d, n_restarts, ks_in, *p, seeded(*p, seeds),
+                       {nullptr, nullptr, spectra_dev, ld_out, d->n_cols, n_iter_host, err_host}, stream);
 }
 
 int cnmf_last_timing(cnmf_handle_t h, double* rng_ms, double* h2d_ms, double* solve_ms, double* d2h_ms) {
@@ -644,24 +719,8 @@ int cnmf_factorize_init(cnmf_dataset_t d, int n_restarts, const int32_t* ks_in, 
                         int32_t* n_iter_host, double* err_host, void* stream) {
   CNMF_TRY(check_params(d, p));
   CNMF_REQUIRE(n_restarts > 0 && ks_in && Wt0_host && H0_host && spectra_host, "factorize_init: bad arguments");
-  cnmf_handle_s* h = d->h;
-  cudaStream_t s = as_stream(stream);
-  CNMF_CUDA_CHECK(cudaSetDevice(h->device));
-  std::vector<int> ks(ks_in, ks_in + n_restarts);
-  int SK = 0;
-  for (int r = 0; r < n_restarts; ++r) {
-    CNMF_REQUIRE(ks[r] >= 1 && ks[r] <= KMAX, "factorize_init: n_components must be in [1, 32] on the CUDA path");
-    SK += ks[r];
-  }
-  FactorBuffers fb;
-  CNMF_TRY(alloc_factors(h, SK, d->ld_r, d->ld_c, p->precision == CNMF_PRECISION_TF32X3, &fb));
-  CNMF_CUDA_CHECK(cudaMemsetAsync(fb.Fr, 0, (size_t)SK * d->ld_r * 4, s));
-  CNMF_CUDA_CHECK(cudaMemsetAsync(fb.Fc, 0, (size_t)SK * d->ld_c * 4, s));
-  CNMF_CUDA_CHECK(cudaMemcpy2DAsync(fb.Fr, (size_t)d->ld_r * 4, Wt0_host, (size_t)d->n_rows * 4, (size_t)d->n_rows * 4,
-                                    SK, cudaMemcpyHostToDevice, s));
-  CNMF_CUDA_CHECK(cudaMemcpy2DAsync(fb.Fc, (size_t)d->ld_c * 4, H0_host, (size_t)d->n_cols * 4, (size_t)d->n_cols * 4,
-                                    SK, cudaMemcpyHostToDevice, s));
-  return run_and_download(d, ks, SK, fb, *p, spectra_host, usages_host, n_iter_host, err_host, s);
+  return factorize_run(d, n_restarts, ks_in, *p, {Starts::HOST_FACTORS, nullptr, Wt0_host, H0_host},
+                       {spectra_host, usages_host, nullptr, 0, 0, n_iter_host, err_host}, stream);
 }
 
 int cnmf_factorize_dev(cnmf_dataset_t d, int n_restarts, const int32_t* ks_in, const float* Wt0_dev,
@@ -669,62 +728,18 @@ int cnmf_factorize_dev(cnmf_dataset_t d, int n_restarts, const int32_t* ks_in, c
                        double* err_host, void* stream) {
   CNMF_TRY(check_params(d, p));
   CNMF_REQUIRE(n_restarts > 0 && ks_in && Wt0_dev && H0_dev && spectra_dev, "factorize_dev: bad arguments");
-  cnmf_handle_s* h = d->h;
-  cudaStream_t s = as_stream(stream);
-  CNMF_CUDA_CHECK(cudaSetDevice(h->device));
-  std::vector<int> ks(ks_in, ks_in + n_restarts);
-  int SK = 0;
-  for (int r = 0; r < n_restarts; ++r) {
-    CNMF_REQUIRE(ks[r] >= 1 && ks[r] <= KMAX, "factorize_dev: n_components must be in [1, 32] on the CUDA path");
-    SK += ks[r];
-  }
-  const bool tf32 = p->precision == CNMF_PRECISION_TF32X3;
-  FactorBuffers fb;
-  CNMF_TRY(alloc_factors(h, SK, d->ld_r, d->ld_c, tf32, &fb));
-  CNMF_CUDA_CHECK(cudaMemcpyAsync(fb.Fr, Wt0_dev, (size_t)SK * d->ld_r * 4, cudaMemcpyDeviceToDevice, s));
-  CNMF_CUDA_CHECK(cudaMemcpyAsync(fb.Fc, H0_dev, (size_t)SK * d->ld_c * 4, cudaMemcpyDeviceToDevice, s));
-  DataView v = make_view(d, false);
-  if (tf32 && !v.f16) {      // f16 datasets: the solver emits fp16 pieces itself; tf32 pieces would be dead work
-    CNMF_TRY(launch_split_scaled(fb.Fr, fb.Fr_hi, fb.Fr_lo, SK, d->ld_r, v.exact ? v.scale_r : nullptr, s));
-    CNMF_TRY(launch_split_scaled(fb.Fc, fb.Fc_hi, fb.Fc_lo, SK, d->ld_c, v.exact ? v.scale_c : nullptr, s));
-    h->launches += 2;
-  }
-  SolveIO io;
-  io.R = n_restarts;
-  io.ks = ks;
-  io.Fr = fb.Fr; io.Fr_hi = fb.Fr_hi; io.Fr_lo = fb.Fr_lo;
-  io.Fc = fb.Fc; io.Fc_hi = fb.Fc_hi; io.Fc_lo = fb.Fc_lo;
-  io.update_cols = true;
-  CNMF_TRY(solve_batched(h, v, io, *p, s));
-  CNMF_CUDA_CHECK(cudaMemcpyAsync(spectra_dev, fb.Fc, (size_t)SK * d->ld_c * 4, cudaMemcpyDeviceToDevice, s));
-  CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
-  for (int r = 0; r < n_restarts; ++r) {
-    if (n_iter_host) n_iter_host[r] = io.n_iter[r];
-    if (err_host) err_host[r] = io.err[r];
-  }
-  return 0;
+  return factorize_run(d, n_restarts, ks_in, *p, {Starts::DEVICE_FACTORS, nullptr, Wt0_dev, H0_dev},
+                       {nullptr, nullptr, spectra_dev, d->ld_c, d->ld_c, n_iter_host, err_host}, stream);
 }
 
 int cnmf_random_init_dev(cnmf_dataset_t d, int n_restarts, const int32_t* ks_in, const uint32_t* seeds, float* Wt_dev,
                          float* H_dev, void* stream) {
   CNMF_REQUIRE(d && n_restarts > 0 && ks_in && seeds && Wt_dev && H_dev, "random_init_dev: bad arguments");
-  cnmf_handle_s* h = d->h;
   cudaStream_t s = as_stream(stream);
-  CNMF_CUDA_CHECK(cudaSetDevice(h->device));
-  std::vector<int> ks(ks_in, ks_in + n_restarts), off(n_restarts);
-  std::vector<double> avgs(n_restarts);
-  const double mean_d = d->sum / ((double)d->n_rows * (double)d->n_cols);
-  int SK = 0;
-  for (int r = 0; r < n_restarts; ++r) {
-    CNMF_REQUIRE(ks[r] >= 1 && ks[r] <= KMAX, "random_init_dev: n_components must be in [1, 32]");
-    off[r] = SK;
-    SK += ks[r];
-    avgs[r] = std::sqrt(mean_d / ks[r]);
-  }
-  CNMF_CUDA_CHECK(cudaMemsetAsync(Wt_dev, 0, (size_t)SK * d->ld_r * 4, s));
-  CNMF_CUDA_CHECK(cudaMemsetAsync(H_dev, 0, (size_t)SK * d->ld_c * 4, s));
-  CNMF_TRY(launch_rng_init(seeds, ks.data(), off.data(), avgs.data(), n_restarts, d->n_rows, d->n_cols, Wt_dev, d->ld_r,
-                           H_dev, d->ld_c, h, s));
+  CNMF_CUDA_CHECK(cudaSetDevice(d->h->device));
+  RestartTable t;
+  CNMF_TRY(restart_table(d, n_restarts, ks_in, &t));
+  CNMF_TRY(device_rng(d, t, seeds, Wt_dev, H_dev, s));
   CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
   return 0;
 }
@@ -737,19 +752,3 @@ int cnmf_dataset_ld(cnmf_dataset_t d, int* ld_rows, int* ld_cols) {
 }
 
 }  // extern "C"
-
-namespace cnmf {
-
-int dataset_ensure_full_transpose(cnmf_dataset_s* d, cudaStream_t s) {
-  if (d->Xt) return 0;
-  CNMF_CUDA_CHECK(cudaSetDevice(d->h->device));
-  const size_t nxt = (size_t)d->n_cols * d->ld_r;
-  CNMF_TRY(cnmf_dataset_alloc_internal(d, &d->Xt, nxt));
-  CNMF_CUDA_CHECK(cudaMemsetAsync(d->Xt, 0, nxt * sizeof(float), s));
-  CNMF_TRY(launch_transpose(d->X, d->n_rows, d->n_cols, d->ld_c, d->Xt, nullptr, nullptr, d->ld_r, s));
-  d->h->launches += 1;
-  CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
-  return 0;
-}
-
-}  // namespace cnmf

@@ -13,12 +13,6 @@
 
 using namespace cnmf;
 
-#define CNMF_TRY(expr)            \
-  do {                            \
-    int _rc = (expr);             \
-    if (_rc != 0) return _rc;     \
-  } while (0)
-
 namespace {
 
 __global__ void fill_kernel(float* p, float v, int rows, int n, int ld) {
@@ -98,6 +92,21 @@ __global__ void gather_cols_kernel(const float* __restrict__ src, int rows, int 
   for (int r = blockIdx.y; r < rows; r += gridDim.y) dst[(long long)r * ld_dst + c] = src[(long long)r * ld_src + sc] * f;
 }
 
+// out (M x N, row stride N) = the sum in fp64 of the `slices` split-K slices of the device GEMM output C (M x ldc each,
+// contiguous); synchronises the stream
+int download_split_sum(const float* C, int slices, int M, int N, int ldc, float* out, cudaStream_t s) {
+  std::vector<float> tmp((size_t)slices * M * ldc);
+  CNMF_CUDA_CHECK(cudaMemcpyAsync(tmp.data(), C, tmp.size() * 4, cudaMemcpyDeviceToHost, s));
+  CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
+  for (int m = 0; m < M; ++m)
+    for (int n = 0; n < N; ++n) {
+      double a = 0.0;
+      for (int z = 0; z < slices; ++z) a += tmp[(size_t)z * M * ldc + (size_t)m * ldc + n];
+      out[(size_t)m * N + n] = (float)a;
+    }
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -159,10 +168,6 @@ int cnmf_dataset_row_sums(cnmf_dataset_t d, double* row_sums_host, void* stream)
   return 0;
 }
 
-// defined in capi.cu (internal; not in the public header)
-int cnmf_dataset_finish_internal(cnmf_dataset_t d, void* stream);
-int cnmf_dataset_alloc_internal(cnmf_dataset_t d, float** p, size_t elems);
-
 int cnmf_dataset_from_columns(cnmf_dataset_t src, const int32_t* cols_host, const float* col_scale_host, int n_cols,
                               void* stream, cnmf_dataset_t* out) {
   CNMF_REQUIRE(src && cols_host && col_scale_host && out && n_cols > 0, "dataset_from_columns: bad arguments");
@@ -176,20 +181,9 @@ int cnmf_dataset_from_columns(cnmf_dataset_t src, const int32_t* cols_host, cons
   if (!d_cols || !d_scale) return -2;
   CNMF_CUDA_CHECK(cudaMemcpyAsync(d_cols, cols_host, sizeof(int) * n_cols, cudaMemcpyHostToDevice, s));
   CNMF_CUDA_CHECK(cudaMemcpyAsync(d_scale, col_scale_host, sizeof(float) * n_cols, cudaMemcpyHostToDevice, s));
-  auto* d = new cnmf_dataset_s();
-  d->h = h;
-  d->n_rows = src->n_rows;
-  d->n_cols = n_cols;
-  d->ld_c = pad_ld(n_cols);
-  d->ld_r = pad_ld(src->n_rows);
-  d->precision = src->precision;
-  d->allow_exact = src->allow_exact;
-  d->want_f16 = src->want_f16;
-  int rc = cnmf_dataset_alloc_internal(d, &d->X, (size_t)d->n_rows * d->ld_c);
-  if (rc == 0) {
-    cudaError_t e = cudaMemsetAsync(d->X, 0, (size_t)d->n_rows * d->ld_c * sizeof(float), s);
-    if (e != cudaSuccess) rc = -2;
-  }
+  cnmf_dataset_s* d = nullptr;
+  CNMF_TRY(dataset_new(h, src, 0, src->n_rows, n_cols, &d));
+  int rc = cudaMemsetAsync(d->X, 0, (size_t)d->n_rows * d->ld_c * sizeof(float), s) == cudaSuccess ? 0 : -2;
   if (rc == 0) {
     dim3 grid((n_cols + 127) / 128, std::min(d->n_rows, 16384));
     gather_cols_kernel<<<grid, 128, 0, s>>>(src->X, d->n_rows, src->ld_c, d_cols, d_scale, n_cols, d->X, d->ld_c);
@@ -200,25 +194,19 @@ int cnmf_dataset_from_columns(cnmf_dataset_t src, const int32_t* cols_host, cons
     // an exact-count source stays exact: same integer matrix (the selected columns), same row scale, and the
     // column scale becomes scale[c] * src.col_scale[cols[c]]; finish() rebuilds C from the scaled values
     d->exact = true;
-    rc = cnmf_dataset_alloc_internal(d, &d->col_scale, (size_t)d->ld_c);
+    rc = dataset_alloc(d, &d->col_scale, (size_t)d->ld_c);
     if (rc == 0) {
       combine_scale_kernel<<<(d->ld_c + 255) / 256, 256, 0, s>>>(d_scale, src->col_scale, d_cols, n_cols, d->ld_c, d->col_scale);
       h->launches += 1;
       if (cudaGetLastError() != cudaSuccess) rc = -2;
     }
     if (rc == 0 && src->row_scale) {
-      rc = cnmf_dataset_alloc_internal(d, &d->row_scale, (size_t)d->ld_r);
+      rc = dataset_alloc(d, &d->row_scale, (size_t)d->ld_r);
       if (rc == 0 && cudaMemcpyAsync(d->row_scale, src->row_scale, sizeof(float) * d->ld_r, cudaMemcpyDeviceToDevice, s) != cudaSuccess)
         rc = -2;
     }
   }
-  if (rc == 0) rc = cnmf_dataset_finish_internal(d, stream);
-  if (rc != 0) {
-    cnmf_dataset_destroy(d);
-    return rc;
-  }
-  *out = d;
-  return 0;
+  return finish_or_destroy(d, rc, s, out);
 }
 
 int cnmf_dataset_scale_rows(cnmf_dataset_t src, const float* row_scale_host, void* stream, cnmf_dataset_t* out) {
@@ -229,29 +217,12 @@ int cnmf_dataset_scale_rows(cnmf_dataset_t src, const float* row_scale_host, voi
   float* d_rs = static_cast<float*>(h->dev_buf("scalerows.rs", sizeof(float) * src->n_rows));
   if (!d_rs) return -2;
   CNMF_CUDA_CHECK(cudaMemcpyAsync(d_rs, row_scale_host, sizeof(float) * src->n_rows, cudaMemcpyHostToDevice, s));
-  auto* d = new cnmf_dataset_s();
-  d->h = h;
-  d->n_rows = src->n_rows;
-  d->n_cols = src->n_cols;
-  d->ld_c = src->ld_c;
-  d->ld_r = src->ld_r;
-  d->precision = src->precision;
-  d->allow_exact = src->allow_exact;
-  d->want_f16 = src->want_f16;
-  int rc = cnmf_dataset_alloc_internal(d, &d->X, (size_t)d->n_rows * d->ld_c);
-  if (rc == 0) {
-    scale_rows_kernel<<<148 * 8, 256, 0, s>>>(src->X, d->n_rows, d->n_cols, d->ld_c, d_rs, d->X);
-    h->launches += 1;
-    if (cudaGetLastError() != cudaSuccess) rc = -2;
-  }
+  cnmf_dataset_s* d = nullptr;
+  CNMF_TRY(dataset_new(h, src, 0, src->n_rows, src->n_cols, &d));
+  scale_rows_kernel<<<148 * 8, 256, 0, s>>>(src->X, d->n_rows, d->n_cols, d->ld_c, d_rs, d->X);
+  h->launches += 1;
   // exact-count detection runs from scratch in finish(): counts x (1e6 / cell total) is again scaled integers
-  if (rc == 0) rc = cnmf_dataset_finish_internal(d, stream);
-  if (rc != 0) {
-    cnmf_dataset_destroy(d);
-    return rc;
-  }
-  *out = d;
-  return 0;
+  return finish_or_destroy(d, cudaGetLastError() == cudaSuccess ? 0 : -2, s, out);
 }
 
 // --------------------------------------------------------------------------------- refit
@@ -268,21 +239,12 @@ int cnmf_refit(cnmf_dataset_t d, int transposed, int k, const float* fixed_host,
   if (p->beta_loss != CNMF_LOSS_FROBENIUS) CNMF_TRY(dataset_ensure_full_transpose(d, s));
   DataView v = make_view(d, transposed != 0);
 
-  const size_t nr = (size_t)k * v.ld_r, nc = (size_t)k * v.ld_c;
-  float* Fr = static_cast<float*>(h->dev_buf("refit.Fr", nr * 4));
-  float* Fc = static_cast<float*>(h->dev_buf("refit.Fc", nc * 4));
-  float *Fr_hi = nullptr, *Fr_lo = nullptr, *Fc_hi = nullptr, *Fc_lo = nullptr;
-  if (!Fr || !Fc) return -2;
-  if (tf32) {
-    Fr_hi = static_cast<float*>(h->dev_buf("refit.Fr_hi", nr * 4));
-    Fr_lo = static_cast<float*>(h->dev_buf("refit.Fr_lo", nr * 4));
-    Fc_hi = static_cast<float*>(h->dev_buf("refit.Fc_hi", nc * 4));
-    Fc_lo = static_cast<float*>(h->dev_buf("refit.Fc_lo", nc * 4));
-    if (!Fr_hi || !Fr_lo || !Fc_hi || !Fc_lo) return -2;
-  }
-  CNMF_CUDA_CHECK(cudaMemsetAsync(Fr, 0, nr * 4, s));
-  CNMF_CUDA_CHECK(cudaMemsetAsync(Fc, 0, nc * 4, s));
-  CNMF_CUDA_CHECK(cudaMemcpy2DAsync(Fc, (size_t)v.ld_c * 4, fixed_host, (size_t)v.n_c * 4, (size_t)v.n_c * 4, k,
+  SolveIO io;
+  CNMF_TRY(alloc_factors(h, "refit.", k, v.ld_r, v.ld_c, tf32, &io));
+  float* Fr = io.Fr;
+  CNMF_CUDA_CHECK(cudaMemsetAsync(Fr, 0, (size_t)k * v.ld_r * 4, s));
+  CNMF_CUDA_CHECK(cudaMemsetAsync(io.Fc, 0, (size_t)k * v.ld_c * 4, s));
+  CNMF_CUDA_CHECK(cudaMemcpy2DAsync(io.Fc, (size_t)v.ld_c * 4, fixed_host, (size_t)v.n_c * 4, (size_t)v.n_c * 4, k,
                                     cudaMemcpyHostToDevice, s));
   if (p->solver == CNMF_SOLVER_MU) {
     // sklearn _nmf.py:1223-1226: W = full(sqrt(X.mean() / k))
@@ -291,16 +253,9 @@ int cnmf_refit(cnmf_dataset_t d, int transposed, int k, const float* fixed_host,
     CNMF_CUDA_CHECK(cudaGetLastError());
     h->launches += 1;
   }  // 'cd': zeros (sklearn _nmf.py:1227-1228)
-  if (tf32 && !v.f16) {
-    CNMF_TRY(launch_split_scaled(Fr, Fr_hi, Fr_lo, k, v.ld_r, v.exact ? v.scale_r : nullptr, s));
-    CNMF_TRY(launch_split_scaled(Fc, Fc_hi, Fc_lo, k, v.ld_c, v.exact ? v.scale_c : nullptr, s));
-    h->launches += 2;
-  }
-  SolveIO io;
+  CNMF_TRY(split_factors(h, v, io, k, tf32, s));
   io.R = 1;
   io.ks = {k};
-  io.Fr = Fr; io.Fr_hi = Fr_hi; io.Fr_lo = Fr_lo;
-  io.Fc = Fc; io.Fc_hi = Fc_hi; io.Fc_lo = Fc_lo;
   io.update_cols = false;
   auto t_solve = std::chrono::steady_clock::now();
   if (h->profile) {
@@ -357,9 +312,6 @@ int cnmf_project_rows(cnmf_dataset_t d, int k, const float* Ut_host, float* out_
     }
     h->launches += 1;
   }
-  GemmArgs g{};
-  g.M = k; g.N = d->n_cols; g.Kd = d->n_rows;
-  g.lda = d->ld_r; g.ldb = d->ld_r; g.ldc = d->ld_c;
   int splits = 1;
   {
     const int tiles = ((k + 127) / 128) * ((d->n_cols + 255) / 256);
@@ -368,37 +320,12 @@ int cnmf_project_rows(cnmf_dataset_t d, int k, const float* Ut_host, float* out_
     splits = std::min(splits, 32);
     splits = gemm_effective_splits(d->n_rows, splits, d->f16 ? 1 : 0);
   }
-  g.splits = g.splits_effective = splits;
-  g.c_split_stride = (long long)k * d->ld_c;
   float* C = static_cast<float*>(h->dev_buf("proj.C", (size_t)splits * k * d->ld_c * 4));
   if (!C) return -2;
-  g.C = C;
-  if (tf32) {
-    g.A_hi = A_hi; g.A_lo = A_lo; g.B_hi = d->Xt_hi; g.B_lo = d->Xt_lo;
-    g.b_exact = d->exact ? 1 : 0;
-    g.out_col_scale = d->exact ? d->col_scale : nullptr;
-    if (d->f16) {
-      g.f16 = 1;
-      g.B_hi = static_cast<const float*>(d->Xt_h16);
-      g.a_tile_scale = A_rs;
-      g.a_tiles = a_tiles;
-    }
-    CNMF_TRY(gemm_tf32x3(g, s));
-  } else {
-    g.A_hi = A; g.B_hi = d->Xt;
-    CNMF_TRY(gemm_fp32_simt(g, s));
-  }
+  CNMF_TRY(gemm_run(tf32, d->exact, d->col_scale, k, {A, A_hi, A_lo, A_rs, d->ld_r}, make_view(d, false).B_cols, C,
+                    d->ld_c, {splits, 0, (long long)k * d->ld_c}, s));
   h->launches += 1;
-  std::vector<float> tmp((size_t)splits * k * d->ld_c);
-  CNMF_CUDA_CHECK(cudaMemcpyAsync(tmp.data(), C, tmp.size() * 4, cudaMemcpyDeviceToHost, s));
-  CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
-  for (int c = 0; c < k; ++c)
-    for (int j = 0; j < d->n_cols; ++j) {
-      double a = 0.0;
-      for (int z = 0; z < splits; ++z) a += tmp[(size_t)z * k * d->ld_c + (size_t)c * d->ld_c + j];
-      out_host[(size_t)c * d->n_cols + j] = (float)a;
-    }
-  return 0;
+  return download_split_sum(C, splits, k, d->n_cols, d->ld_c, out_host, s);
 }
 
 // --------------------------------------------------------------------------------- raw GEMM hook
@@ -427,35 +354,32 @@ int cnmf_gemm_abt_host(cnmf_handle_t h, int precision, const float* A, const flo
   CNMF_TRY(launch_split_tf32(dA, dAh, dAl, (long long)na, s));
   CNMF_TRY(launch_split_tf32(dB, dBh, dBl, (long long)nb, s));
   CNMF_CUDA_CHECK(cudaMemsetAsync(dC, 0xff, (size_t)se * M * ldc * 4, s));   // NaN pattern: unwritten outputs show up
-  GemmArgs g{};
-  g.M = M; g.N = N; g.Kd = Kd; g.lda = lda; g.ldb = lda; g.ldc = ldc;
-  g.C = dC; g.c_split_stride = (long long)M * ldc; g.splits = splits; g.splits_effective = se;
   const bool f16 = precision == CNMF_PRECISION_F16X2;    // B must hold integers <= 2048 (exact in fp16)
+  const int tiles = (lda + 511) / 512;
+  float* dRs = nullptr;
   if (f16) {
-    const int tiles = (lda + 511) / 512;
-    float* dRs = static_cast<float*>(h->dev_buf("gemmtest.rs", sizeof(float) * (size_t)M * tiles));
+    dRs = static_cast<float*>(h->dev_buf("gemmtest.rs", sizeof(float) * (size_t)M * tiles));
     if (!dRs) return -2;
     CNMF_TRY(launch_emit_f16(dA, M, Kd, lda, nullptr, dAh, dAl, dRs, tiles, s));
     CNMF_TRY(launch_to_half(dB, dBh, (long long)nb, s));
-    g.A_hi = dAh; g.A_lo = dAl; g.B_hi = dBh; g.b_exact = 1; g.f16 = 1; g.a_tile_scale = dRs; g.a_tiles = tiles;
-  } else if (precision == CNMF_PRECISION_TF32X3) { g.A_hi = dAh; g.A_lo = dAl; g.B_hi = dBh; g.B_lo = dBl; }
-  else { g.A_hi = dA; g.B_hi = dB; }
+  }
   const bool tc = f16 || precision == CNMF_PRECISION_TF32X3;
+  const GemmA a{dA, dAh, dAl, dRs, lda};
+  const Operand b{dB, dBh, f16 ? nullptr : dBl, f16 ? dBh : nullptr, N, Kd, lda};
+  auto gemm = [&] { return gemm_run(tc, f16, nullptr, M, a, b, dC, ldc, {se, 0, (long long)M * ldc}, s); };
   cudaEvent_t e0, e1;
   CNMF_CUDA_CHECK(cudaEventCreate(&e0));
   CNMF_CUDA_CHECK(cudaEventCreate(&e1));
   if (reps < 1) reps = 1;
-  int rc = tc ? gemm_tf32x3(g, s) : gemm_fp32_simt(g, s);   // warm-up + result
+  int rc = gemm();   // warm-up + result
   if (rc == 0 && reps > 1) {
     cudaEventRecord(e0, s);
-    for (int i = 0; i < reps && rc == 0; ++i) rc = tc ? gemm_tf32x3(g, s) : gemm_fp32_simt(g, s);
+    for (int i = 0; i < reps && rc == 0; ++i) rc = gemm();
     cudaEventRecord(e1, s);
   }
   h->launches += reps;
   if (rc != 0) return rc;
-  std::vector<float> tmp((size_t)se * M * ldc);
-  CNMF_CUDA_CHECK(cudaMemcpyAsync(tmp.data(), dC, tmp.size() * 4, cudaMemcpyDeviceToHost, s));
-  CNMF_CUDA_CHECK(cudaStreamSynchronize(s));
+  CNMF_TRY(download_split_sum(dC, se, M, N, ldc, C, s));
   if (ms_out) {
     float ms = 0.f;
     if (reps > 1) cudaEventElapsedTime(&ms, e0, e1);
@@ -463,12 +387,6 @@ int cnmf_gemm_abt_host(cnmf_handle_t h, int precision, const float* A, const flo
   }
   cudaEventDestroy(e0);
   cudaEventDestroy(e1);
-  for (int m = 0; m < M; ++m)
-    for (int n = 0; n < N; ++n) {
-      double a = 0.0;
-      for (int z = 0; z < se; ++z) a += tmp[(size_t)z * M * ldc + (size_t)m * ldc + n];
-      C[(size_t)m * N + n] = (float)a;
-    }
   return 0;
 }
 

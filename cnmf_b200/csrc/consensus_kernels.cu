@@ -13,12 +13,6 @@
 
 using namespace cnmf;
 
-#define CNMF_TRY(expr)            \
-  do {                            \
-    int _rc = (expr);             \
-    if (_rc != 0) return _rc;     \
-  } while (0)
-
 namespace {
 
 template <typename T>

@@ -8,6 +8,7 @@
 
 #include "../../include/cnmf_b200.h"
 #include "common.cuh"
+#include "gemm.h"
 
 struct cnmf_handle_s {
   int device = 0;
@@ -15,9 +16,6 @@ struct cnmf_handle_s {
   long long launches = 0;                       // kernels launched by this library (bench: gpu_launches)
   // optional per-launch timing of the hot kernels (batched GEMM, fused update) with CUDA events on the
   // launching stream; read back by bench.py for the roofline lines
-  // auxiliary stream + events (kept for experiments that co-schedule streaming kernels under a GEMM)
-  cudaStream_t aux = nullptr;
-  cudaEvent_t ev_upd = nullptr, ev_gram = nullptr;
   bool profile = false;
   std::vector<cudaEvent_t> ev_pool;
   struct Pending { int begin; int end; int cls; double work; };   // indices of the start / end events in ev_pool
@@ -32,7 +30,7 @@ struct cnmf_handle_s {
   static constexpr int PROF_CLASSES = 2;
   double prof_ms[PROF_CLASSES] = {0.0, 0.0}, prof_work[PROF_CLASSES] = {0.0, 0.0};
   long long prof_launches[PROF_CLASSES] = {0, 0};
-  double t_rng_ms = 0, t_h2d_ms = 0, t_solve_ms = 0, t_d2h_ms = 0;   // host wall-clock phases of the last cnmf_factorize
+  double t_rng_ms = 0, t_h2d_ms = 0, t_solve_ms = 0, t_d2h_ms = 0;   // host wall-clock phases of the last factorize
   int prof_begin(cudaStream_t s, double work, int cls = 0);    // start event (recorded or shared); returns slot or -1
   void prof_end(cudaStream_t s, int slot);
   void prof_collect();                              // after a stream sync: fold pending pairs into the totals
@@ -82,14 +80,6 @@ namespace cnmf {
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
-struct Operand {     // a K-major matrix as the GEMM sees it
-  const float* full;
-  const float* hi;     // tf32 hi piece, or the exact integer matrix when `exact`
-  const float* lo;
-  const void* h16;     // the exact integer matrix as fp16 (f16x2 datasets), else nullptr
-  int rows, cols, ld;
-};
-
 // View of a dataset for one solve: "rows" are the items of the row factor (Fr: SK x n_r),
 // "cols" the items of the column factor (Fc: SK x n_c).  transposed swaps the roles.
 struct DataView {
@@ -117,6 +107,13 @@ struct SolveIO {
   std::vector<double> err;  // out: final ||X - Fr^T Fc||_F
 };
 
+// Device buffers for SK packed rows of both factors, plus their tf32 pieces when `tf32`, into io.  The buffers are the
+// handle's workspace entries prefix + "Fr", "Fr_hi", ...: each caller keeps its own by its prefix.
+int alloc_factors(cnmf_handle_s* h, const char* prefix, int SK, int ld_r, int ld_c, bool tf32, SolveIO* io);
+// tf32 pieces of both factors with the view's scales folded in (exact datasets).  Nothing to do unless `tf32`, nor for
+// f16 datasets: the solver emits fp16 pieces itself, tf32 pieces would be dead work.
+int split_factors(cnmf_handle_s* h, const DataView& v, const SolveIO& io, int SK, bool tf32, cudaStream_t s);
+
 // Runs the batched solver in place on io.Fr / io.Fc.
 int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_nmf_params& p, cudaStream_t s);
 // beta_loss = kullback-leibler / itakura-saito (nmf_beta.cu); reached through solve_batched
@@ -125,5 +122,16 @@ int matrix_min(cnmf_handle_s* h, const float* X, int rows, int cols, int ld, flo
 // the streaming beta-divergence kernels read X in both orientations in full fp32: builds d->Xt if the dataset
 // (tf32x3 mode) only holds the pieces
 int dataset_ensure_full_transpose(cnmf_dataset_s* d, cudaStream_t s);
+
+// A new dataset of n_rows x n_cols on h with X allocated (contents undefined).  Its precision settings are copied from
+// `like`, or derived from the CNMF_PRECISION_* code `precision` when `like` is nullptr.
+int dataset_new(cnmf_handle_s* h, const cnmf_dataset_s* like, int precision, int n_rows, int n_cols,
+                cnmf_dataset_s** out);
+// device memory owned by d (from the handle's pool), at least 64 floats
+int dataset_alloc(cnmf_dataset_s* d, float** p, size_t elems);
+// builds Xt / tf32 pieces / sums from d->X (already resident, padding zeroed)
+int dataset_finish(cnmf_dataset_s* d, cudaStream_t s);
+// the last step of every dataset constructor: dataset_finish when rc == 0, *out = d on success, d destroyed on failure
+int finish_or_destroy(cnmf_dataset_s* d, int rc, cudaStream_t s, cnmf_dataset_t* out);
 
 }  // namespace cnmf

@@ -45,4 +45,32 @@ int gemm_tf32x3(const GemmArgs& g, cudaStream_t stream);
 // plain fp32 FFMA path (gemm_simt.cu): A = A_hi, B = B_hi exactly; same split-K contract
 int gemm_fp32_simt(const GemmArgs& g, cudaStream_t stream);
 
+struct Operand {     // a K-major matrix as the GEMM sees it
+  const float* full;
+  const float* hi;     // tf32 hi piece, or the exact integer matrix when `exact`
+  const float* lo;
+  const void* h16;     // the exact integer matrix as fp16 (f16x2 datasets), else nullptr
+  int rows, cols, ld;
+};
+
+struct GemmA {       // the M x Kd factor operand (row stride ld)
+  const float* full;         // fp32 path
+  const float* hi;           // tcgen05 path: tf32 pieces, or two fp16 pieces when B.h16 is set
+  const float* lo;
+  const float* tile_scale;   // fp16 pieces: scale per (row, group of 512 reduction elements)
+  int ld;
+};
+
+struct GemmPlan {
+  int splits;               // split-K factor, already effective (gemm_effective_splits)
+  int bn;                   // tile width for the tcgen05 kernel (0 = let the launcher choose)
+  long long split_stride;   // elements between the split-K slices of C
+};
+
+// C[z] (M x B.rows) = A (M x B.cols) * B^T.  tc: tcgen05 on the pieces -- b_exact: B.hi holds B exactly (2 passes) and
+// C[:, n] *= out_col_scale[n] when that is set; B.h16 set: kind::f16 on the fp16 pieces.  Otherwise FFMA on A.full,
+// B.full.  Launches one kernel; counting and profiling it is the caller's.
+int gemm_run(bool tc, bool b_exact, const float* out_col_scale, int M, const GemmA& A, const Operand& B, float* C,
+             int ldc, const GemmPlan& plan, cudaStream_t s);
+
 }  // namespace cnmf

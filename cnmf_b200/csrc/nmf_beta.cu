@@ -380,12 +380,6 @@ __global__ void __launch_bounds__(256) matrix_min_kernel(const float* __restrict
   }
 }
 
-#define CNMF_TRY(expr)            \
-  do {                            \
-    int _rc = (expr);             \
-    if (_rc != 0) return _rc;     \
-  } while (0)
-
 }  // namespace
 
 int matrix_min(cnmf_handle_s* h, const float* X, int rows, int cols, int ld, float* out_host, cudaStream_t s) {

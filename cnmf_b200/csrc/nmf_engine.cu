@@ -41,51 +41,15 @@ DataView make_view(const cnmf_dataset_s* d, bool transposed) {
 
 namespace {
 
-struct GemmPlan {
-  int splits;
-  int bn;                   // tile width for the tcgen05 kernel (0 = let the launcher choose)
-  long long split_stride;   // elements
-};
-
-// C[z] (SK x N) = A (SK x Kd) * B (N x Kd)^T
-int run_gemm(cnmf_handle_s* h, int precision, const float* A, const float* A_hi, const float* A_lo, int SK, int lda,
-             const Operand& B, float* C, int ldc, const GemmPlan& plan, bool exact, const float* out_scale,
-             bool f16, const float* a_tile_scale, cudaStream_t s) {
-  GemmArgs g{};
-  g.M = SK; g.N = B.rows; g.Kd = B.cols;
-  g.lda = lda; g.ldb = B.ld; g.ldc = ldc;
-  g.C = C;
-  g.c_split_stride = plan.split_stride;
-  g.splits = plan.splits;
-  g.splits_effective = plan.splits;
-  g.bn = plan.bn;
+// C[z] (SK x B.rows) = A (SK x B.cols) * B^T, counted and profiled as one GEMM launch
+int run_gemm(cnmf_handle_s* h, bool tc, const GemmA& A, int SK, const Operand& B, float* C, int ldc,
+             const GemmPlan& plan, bool exact, const float* out_scale, cudaStream_t s) {
   h->launches += 1;
-  const int slot = h->prof_begin(s, 2.0 * (double)g.M * (double)g.N * (double)g.Kd);
-  int rc;
-  if (precision == CNMF_PRECISION_TF32X3) {
-    g.A_hi = A_hi; g.A_lo = A_lo; g.B_hi = B.hi; g.B_lo = B.lo;
-    g.b_exact = exact ? 1 : 0;
-    g.out_col_scale = exact ? out_scale : nullptr;
-    if (f16) {       // A_hi / A_lo hold the two fp16 pieces of the row-normalised factor, B its fp16 integer matrix
-      g.f16 = 1;
-      g.B_hi = static_cast<const float*>(B.h16);
-      g.a_tile_scale = a_tile_scale;
-      g.a_tiles = (lda + 511) / 512;
-    }
-    rc = gemm_tf32x3(g, s);
-  } else {
-    g.A_hi = A; g.A_lo = nullptr; g.B_hi = B.full; g.B_lo = nullptr;
-    rc = gemm_fp32_simt(g, s);
-  }
+  const int slot = h->prof_begin(s, 2.0 * (double)SK * (double)B.rows * (double)B.cols);
+  const int rc = gemm_run(tc, exact, out_scale, SK, A, B, C, ldc, plan, s);
   h->prof_end(s, slot);
   return rc;
 }
-
-#define CNMF_TRY(expr)            \
-  do {                            \
-    int _rc = (expr);             \
-    if (_rc != 0) return _rc;     \
-  } while (0)
 
 }  // namespace
 
@@ -293,12 +257,12 @@ int solve_batched(cnmf_handle_s* h, const DataView& v, SolveIO& io, const cnmf_n
     return launch_finalize(nullptr, nullptr, part, out, chunks, bm(), s);
   };
   auto gemm_rows = [&]() -> int {   // NUM_r = Fc * B_rows^T
-    return run_gemm(h, p.precision, wFc, wFc_hi, wFc_lo, SK, v.ld_c, v.B_rows, NUMr, v.ld_r, plan_r, v.exact, v.scale_r,
-                    f16, d_rs_c, s);
+    return run_gemm(h, tf32, {wFc, wFc_hi, wFc_lo, d_rs_c, v.ld_c}, SK, v.B_rows, NUMr, v.ld_r, plan_r, v.exact,
+                    v.scale_r, s);
   };
   auto gemm_cols = [&]() -> int {   // NUM_c = Fr * B_cols^T
-    return run_gemm(h, p.precision, wFr, wFr_hi, wFr_lo, SK, v.ld_r, v.B_cols, NUMc, v.ld_c, plan_c, v.exact, v.scale_c,
-                    f16, d_rs_r, s);
+    return run_gemm(h, tf32, {wFr, wFr_hi, wFr_lo, d_rs_r, v.ld_r}, SK, v.B_cols, NUMc, v.ld_c, plan_c, v.exact,
+                    v.scale_c, s);
   };
 
   // gathers `cnt` restarts' rows: dst[dst_off[i] ..] <- src[src_off[i] ..].  Index triples go through a pinned

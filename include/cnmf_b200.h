@@ -85,8 +85,10 @@ int cnmf_profile_get(cnmf_handle_t h, double* gemm_ms, long long* gemm_launches,
  * (work = algorithmic bytes: factor read + product slices read + factor and tf32 pieces written) */
 int cnmf_profile_get_class(cnmf_handle_t h, int kernel_class, double* ms, long long* launches, double* work);
 
-/* host wall-clock phases (ms) of the last cnmf_factorize on this handle: host RNG, H2D of the initial
- * factors, batched solve, D2H of the results */
+/* host wall-clock phases (ms) of the last factorize call on this handle (cnmf_factorize, _seeds_dev, _init or _dev;
+ * each resets all four when it starts): host RNG (device RNG: its enqueue time), H2D of the host RNG's factors,
+ * batched solve, copy-out of the results.  A phase the call did not run reads 0.  With profiling enabled,
+ * cnmf_refit and cnmf_kmeans_fit write their own phases into the same fields. */
 int cnmf_last_timing(cnmf_handle_t h, double* rng_ms, double* h2d_ms, double* solve_ms, double* d2h_ms);
 
 /* ---- dataset: a cells x genes matrix made resident on the device ------------------- */
